@@ -10,7 +10,7 @@ Green's-function flux on the wall, SI mu0) around the Picard + multigrid inner s
 the north_star target).  One "step" = one complete batched solve.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--workload free_boundary|fixed_boundary|slab]
-                    [--scaling weak|strong] [--impl reference]
+                    [--scaling weak|strong] [--impl reference] [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = converged equilibria/s with the per-sample inputs already resident in
 HBM; `e2e` = the same metric through the public host API (BatchedFusionKernel.solve_free_boundary: host arrays in,
@@ -26,6 +26,11 @@ oracle (psi rel-L2 <= 1e-9, outer iterations equal, Picard iterations +-1 per in
 
 `--workload slab` is BASELINE configs[4]: ONE 4097^2 multigrid_solve, slab-decomposed over the N ranks (strong
 scaling), GLUPS per V-cycle against the 261 B/point HBM roofline.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned in its last step (rank 0) as
+DIR/<name>.npy in float64: psi, j_phi, psi_ext, summary, fb_summary of the batch (fixed_boundary: psi, j_phi,
+summary; slab: the owned psi rows and residual_linf, cycles, converged).  The inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -57,6 +62,8 @@ ITER_COILS = [(3.5, 3.0, -1.0), (8.0, 3.0, 4.0), (9.5, 0.0, 6.0), (8.0, -3.0, 4.
               (9.5, 3.0, 3.0), (2.1, 0.0, 0.0)]
 PSI_TOL = 1e-9
 BYTES_PER_POINT_ITER = 350.0  # SURVEY.md 8d: 261 (V-cycle, all levels) + 89 (topology, source, relax, residual)
+DUMP_BYTES = 60_000_000  # --dump-outputs stays below 64 MB, .npy headers included
+DUMP_SEED = 0
 
 
 def base_config(n: int = GRID) -> dict:
@@ -265,6 +272,26 @@ def measured_peak_hbm():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+def dump_outputs(out_dir: str, fields: dict, scalars: dict | None = None) -> None:
+    """Write device tensors that share a leading axis (the equilibria of a batch, or the rows of a slab) as
+    <out_dir>/<name>.npy, float64.  When together they exceed DUMP_BYTES, every field keeps the same sorted sample of
+    that axis, drawn with DUMP_SEED, so runs with the same arguments stay comparable entry for entry.  `scalars` are
+    written as 0-d arrays."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    n = next(iter(fields.values())).shape[0]
+    per_entry = sum(t.element_size() * t.numel() // n for t in fields.values())
+    keep = min(n, DUMP_BYTES // per_entry)
+    if keep < 1:
+        raise SystemExit(f"bench.py: one entry of the outputs ({per_entry} B) exceeds the --dump-outputs budget")
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(DUMP_SEED).choice(n, keep, replace=False))
+    for name, t in fields.items():
+        a = t.index_select(0, torch.as_tensor(idx, device=t.device)).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64, copy=False))
+    for name, v in (scalars or {}).items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+
 class _Dist:
     """torch.distributed plumbing (one process per GPU under torchrun); no data-path collective is used by the
     batch workloads - only the barrier and the reductions of the timing / convergence scalars."""
@@ -392,6 +419,8 @@ def run_gpu_arm(args) -> None:
     sampler = ClockSampler(local)
     sampler.start()
     ms, launches, last = dd.timed(step_resident, args.steps, _lib.launch_count)
+    if args.dump_outputs and rank == 0:  # before the legs below reuse psi_buf / j_buf
+        dump_outputs(args.dump_outputs, last)
     summ = last["summary"].cpu().numpy()
     if free_boundary:
         fbs = last["fb_summary"].cpu().numpy()
@@ -622,6 +651,8 @@ def run_slab(args) -> None:
     sampler.stop_flag.set()
     sampler.join(timeout=2)
     psi, res, cycles, conv = out
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"psi": psi}, {"residual_linf": res, "cycles": cycles, "converged": conv})
     if rank == 0:
         peak, peak_src = measured_peak_hbm()
         n_int = (n - 2) ** 2
@@ -670,7 +701,14 @@ def main() -> None:
     ap.add_argument("--no-extras", action="store_true", help="skip the plasma-wall / fixed-boundary / smoother legs")
     ap.add_argument("--slab-nccl", action="store_true", help="slab workload: NCCL point-to-point halos instead of peer memory")
     ap.add_argument("--slab-nccl-gather", action="store_true", help="slab workload: NCCL all-gather of the coarse level (no multi-rank graph)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed path returned in its last step as DIR/<name>.npy (float64, rank 0; a "
+                         "fixed, seeded sample of the equilibria or rows when the whole would exceed 60 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path, not of --impl reference")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.workload == "slab":

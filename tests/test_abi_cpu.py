@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import ctypes
+import hashlib
 import os
 import re
 
@@ -48,6 +49,14 @@ def test_reference_abi_symbols_match_hpc_bridge_contract():
     assert lib.run_step_converged(None, None, None, 0, 1, 1.5, 1e-6, ctypes.byref(d)) == 0
     assert d.value == 0.0
     lib.destroy_solver(None)
+
+
+def test_sha256_sidecar_matches_the_library():
+    """hpc_bridge.py loads a native solver only when <lib>.sha256 holds the file's digest (the Makefile writes it)."""
+    with open(_lib.LIB_PATH, "rb") as f:
+        digest = hashlib.sha256(f.read()).hexdigest()
+    with open(_lib.LIB_PATH + ".sha256") as f:
+        assert f.read().strip() == digest
 
 
 @pytest.mark.parametrize("shape,expect", [
