@@ -226,6 +226,41 @@ int gsb_free_boundary_solve(gsb_ctx *ctx, const gsb_picard_params *p, const gsb_
                             const double *ip_dev, const double *prof_dev, double *jphi_dev, double *summary_dev,
                             double *fb_summary_dev, int batch, void *stream);
 
+typedef struct gsb_shape_params {
+  int n_coils;            /* 1..32 */
+  const double *coil_rz;  /* HOST [n_coils][2] coil (R, Z) */
+  int n_points;           /* shape-control points P, 1..1024 */
+  const double *points;   /* HOST [P][2] (R, Z) of the control points */
+  double alpha;           /* Tikhonov weight (tikhonov_alpha), finite and >= 0 */
+  int isoflux;            /* 1: target = mean of the bilinear samples of the new Psi at the points (broadcast to P);
+                             0: target_dev holds explicit per-equilibrium targets */
+  const double *limits;   /* HOST [n_coils] current limits (> 0; bounds are +-limits) or NULL (unbounded) */
+} gsb_shape_params;
+
+/* solve_free_boundary(optimize_shape=True) (fusion_kernel_free_boundary.py:623-739) for `batch` independent
+ * equilibria on the device.  The outer loop of gsb_free_boundary_solve gains a shape step after each inner Picard
+ * solve of every still-active equilibrium: target t (isoflux mean or explicit), then the coil currents x minimising
+ * |M^T x - t|^2 + alpha |x|^2 within +-limits (M[c][p] = turns_c G_SI(coil c -> point p)), then the coil flux
+ * sum_c x_c turns_c G_c.  The fit is the exact minimiser (bounded-variable least squares on the QR factor of
+ * [M^T; sqrt(alpha) I]), not the stopping point of the reference's interior-point lsq_linear(method="trf"); a
+ * non-finite target or an iteration cap reached keeps the clipped prior currents (the reference's failure path).
+ * A rank-deficient [M^T; sqrt(alpha) I] (alpha = 0 and fewer independent points than coils) fails with GSB_EINVAL
+ * before any Picard launch.
+ * green_dev    [n_coils][nz][nr] si==1 tables of gsb_green_table for these coils
+ * turns_host   HOST [n_coils] integer turns
+ * currents_dev [batch][n_coils] in: starting currents, out: final currents
+ * target_dev   NULL (isoflux) or [batch][P] explicit targets
+ * shape_out_dev [batch][2P+4] out, of each equilibrium's last shape step: target[P], achieved flux M^T x [P],
+ *              rmse, max |achieved - target|, active bounds (|x| within 1e-8 of its limit), fallback (1: prior kept)
+ * psi_ext_dev  [batch][nz][nr] out: coil flux of the final currents
+ * The other arguments are those of gsb_free_boundary_solve. */
+int gsb_free_boundary_shape_solve(gsb_ctx *ctx, const gsb_picard_params *p, const gsb_free_boundary_params *fb,
+                                  const gsb_shape_params *sp, const double *green_dev, const int *turns_host,
+                                  double *currents_dev, const double *target_dev, double *shape_out_dev,
+                                  double *psi_dev, double *psi_ext_dev, const double *wall_m_dev,
+                                  const double *ip_dev, const double *prof_dev, double *jphi_dev, double *summary_dev,
+                                  double *fb_summary_dev, int batch, void *stream);
+
 /* Measurement hook (bench.py roofline): while enabled, gsb_free_boundary_solve brackets every inner Picard solve and
  * every wall GEMM with CUDA events on the launching stream and accumulates
  * out4 = {Picard solves: total ms, count; wall GEMMs: total ms, count}.  out4 may be NULL; reset != 0 zeroes the sums. */

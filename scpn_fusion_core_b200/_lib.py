@@ -36,6 +36,11 @@ class gsb_free_boundary_params(ctypes.Structure):
     _fields_ = [("max_outer_iter", c_int), ("tol", c_double), ("warm_j", c_int)]
 
 
+class gsb_shape_params(ctypes.Structure):
+    _fields_ = [("n_coils", c_int), ("coil_rz", POINTER(c_double)), ("n_points", c_int), ("points", POINTER(c_double)),
+                ("alpha", c_double), ("isoflux", c_int), ("limits", POINTER(c_double))]
+
+
 _dp = POINTER(c_double)
 _ip = POINTER(c_int)
 
@@ -80,6 +85,10 @@ SIGNATURES = {
     "gsb_free_boundary_solve": (c_int, [c_void_p, POINTER(gsb_picard_params), POINTER(gsb_free_boundary_params), c_void_p,
                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int,
                                         c_void_p]),
+    "gsb_free_boundary_shape_solve": (c_int, [c_void_p, POINTER(gsb_picard_params), POINTER(gsb_free_boundary_params),
+                                              POINTER(gsb_shape_params), c_void_p, _ip, c_void_p, c_void_p, c_void_p,
+                                              c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                              c_void_p, c_int, c_void_p]),
     "gsb_enable_peer_access": (c_int, [c_int, c_int]),
     "gsb_ipc_alloc": (c_int, [c_int, c_longlong, POINTER(c_void_p), c_char_p]),
     "gsb_ipc_open": (c_int, [c_int, c_char_p, POINTER(c_void_p)]),

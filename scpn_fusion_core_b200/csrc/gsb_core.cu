@@ -300,6 +300,7 @@ void gsb_destroy(gsb_ctx *ctx) {
   if (ctx->fb_part) cudaFree(ctx->fb_part);
   if (ctx->fb_wall) cudaFree(ctx->fb_wall);
   if (ctx->fb_ints) cudaFree(ctx->fb_ints);
+  if (ctx->fb_shape) cudaFree(ctx->fb_shape);
   if (ctx->h_counter) cudaFreeHost(ctx->h_counter);
   delete ctx;
 }

@@ -357,6 +357,9 @@ struct gsb_ctx {
   // free-boundary outer loop workspace, sized for batch_cap on first use (no allocation in steady state)
   double *fb_old = nullptr, *fb_part = nullptr, *fb_wall = nullptr;
   int *fb_ints = nullptr;
+  // shape-optimising outer loop (gsb_free_boundary_shape_solve): factor, stencil, weights (grow-only)
+  double *fb_shape = nullptr;
+  size_t fb_shape_bytes = 0;
 };
 
 namespace gsb {

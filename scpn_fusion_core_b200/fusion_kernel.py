@@ -673,9 +673,10 @@ class BatchedFusionKernel(_GridMixin):
     def solve_free_boundary(self, coil_currents=None, plasma_current=None, ped_p=None, ped_ff=None, *, turns=None,
                             max_outer_iter: int = 20, tol: float = 1e-4, plasma_wall: bool = False,
                             wall_mu0: float = _MU0_SI, psi0=None, batch: int | None = None, to_host: bool = True,
-                            out: dict | None = None) -> dict[str, Any]:
-        """``FusionKernel.solve_free_boundary(coils, max_outer_iter, tol)`` (fusion_kernel_free_boundary.py:623-739,
-        ``optimize_shape=False``) for B independent equilibria in one device-resident outer loop.
+                            out: dict | None = None, optimize_shape: bool = False, target_points=None,
+                            target_values=None, current_limits=None, tikhonov_alpha: float = 1e-4) -> dict[str, Any]:
+        """``FusionKernel.solve_free_boundary(coils, max_outer_iter, tol, optimize_shape, tikhonov_alpha)``
+        (fusion_kernel_free_boundary.py:623-739) for B independent equilibria in one device-resident outer loop.
 
         coil_currents (B, n_coils) | None (config currents; then give ``batch``), turns (n_coils,) | None (config
         ``turns``, default 1), plasma_current (B,) | None, ped_p / ped_ff (B, 4) | None.  ``plasma_wall=True`` adds
@@ -685,6 +686,17 @@ class BatchedFusionKernel(_GridMixin):
         host tensors (``pinned_outputs``) to receive the fields without a pageable staging copy (see ``solve``).
         Returns per-equilibrium arrays: outer_iterations, final_diff, inner_iterations (sum over the outer
         iterations), fb_converged, plus the keys of ``solve`` for the last inner solve.
+
+        ``optimize_shape=True`` with ``target_points`` (P, 2) re-fits the coil currents to the shape-control points
+        after every inner solve, on the device: target = ``target_values`` ((P,) or (B, P)) or, without them, the mean
+        of the flux sampled at the points (isoflux); currents = argmin |M^T I - target|^2 + tikhonov_alpha |I|^2 within
+        +-``current_limits`` (n_coils,).  The fit is the exact bounded minimiser, where the reference stops
+        ``lsq_linear(method="trf")`` at its tolerance (currents within ~1e-7 relative; a current the reference leaves
+        just inside its limit sits on it here, so ``active_current_bounds`` can be larger).  The result then also has
+        ``coil_currents`` (B, n_coils) and ``shape_optimization`` with the reference's keys (the fit scalars as (B,)
+        arrays, ``target_flux`` / ``achieved_flux`` (B, P)) plus ``fit_fallback`` (B,): the fit failed (non-finite
+        target) and the clipped prior currents were kept, as the reference does.  Without ``target_points`` the call is
+        the ``optimize_shape=False`` solve, like the reference's.
         """
         if max_outer_iter < 1:
             raise ValueError("max_outer_iter must be >= 1.")
@@ -705,31 +717,52 @@ class BatchedFusionKernel(_GridMixin):
         if np.any(np.abs(ip) < 1e-12):
             raise NotImplementedError("zero plasma current samples: use FusionKernel.solve_free_boundary")
         ped = self._ped_rows(B, ped_p, ped_ff)
+        shape = bool(optimize_shape) and target_points is not None
+        spec = self._shape_spec(B, tr, target_points, target_values, current_limits, tikhonov_alpha) if shape else None
         t0 = time.time()
-        w = cc * tr[None, :]  # I * turns (fusion_kernel_free_boundary.py:88-92)
         psi_in = None if psi0 is None else D.to_device(np.asarray(psi0, dtype=np.float64).reshape(B, self.NZ, self.NR),
                                                        self.device)
-        dev = self.solve_free_boundary_device(D.to_device(w, self.device), D.to_device(ip, self.device),
-                                              None if ped is None else D.to_device(ped, self.device),
-                                              max_outer_iter=max_outer_iter, tol=tol, plasma_wall=plasma_wall,
-                                              wall_mu0=wall_mu0, psi_out=psi_in, warm=psi0 is not None)
+        kw = dict(max_outer_iter=max_outer_iter, tol=tol, plasma_wall=plasma_wall, wall_mu0=wall_mu0, psi_out=psi_in,
+                  warm=psi0 is not None)
+        ipd = D.to_device(ip, self.device)
+        pedd = None if ped is None else D.to_device(ped, self.device)
+        if shape:
+            dev = self.solve_free_boundary_device(None, ipd, pedd, optimize_shape=True, target_points=spec["points"],
+                                                  target_values=spec["values"], current_limits=spec["limits"],
+                                                  tikhonov_alpha=spec["alpha"], turns=spec["turns"],
+                                                  currents=D.to_device(cc, self.device), **kw)
+        else:
+            w = cc * tr[None, :]  # I * turns (fusion_kernel_free_boundary.py:88-92)
+            dev = self.solve_free_boundary_device(D.to_device(w, self.device), ipd, pedd, **kw)
         res = self.unpack_summary(dev["summary"].cpu().numpy())
         fb = dev["fb_summary"].cpu().numpy()
         res.update({"outer_iterations": fb[:, 0].astype(np.int64), "final_diff": fb[:, 1],
                     "inner_iterations": fb[:, 2].astype(np.int64), "fb_converged": fb[:, 3] > 0.5})
+        if shape:
+            res["coil_currents"] = dev["currents"].cpu().numpy()
+            res["shape_optimization"] = self._shape_report(spec, dev["shape_out"].cpu().numpy())
         self._fields_to_host(res, dev, to_host, out)
         res["wall_time_s"] = time.time() - t0
         return res
 
     def solve_free_boundary_device(self, w_dev, ip_dev, ped_dev=None, *, max_outer_iter: int = 20, tol: float = 1e-4,
                                    plasma_wall: bool = False, wall_mu0: float = _MU0_SI, psi_out=None, jphi_out=None,
-                                   warm: bool = False, events=None) -> dict[str, Any]:
+                                   warm: bool = False, events=None, optimize_shape: bool = False, target_points=None,
+                                   target_values=None, current_limits=None, tikhonov_alpha: float = 1e-4,
+                                   currents=None, turns=None) -> dict[str, Any]:
         """Device-resident batched free-boundary solve (gsb_free_boundary_solve): w_dev (B, n_coils) = I*turns,
         ip_dev (B,), ped_dev (B, 8) | None - CUDA float64 tensors.  ``psi_out`` is the flux buffer (its content is
         the starting flux when ``warm``, otherwise it is zeroed).  Returns device tensors psi, j_phi, psi_ext,
-        summary (B, 16), fb_summary (B, 4)."""
+        summary (B, 16), fb_summary (B, 4).
+
+        ``optimize_shape=True`` with ``target_points`` (gsb_free_boundary_shape_solve; keywords as in
+        ``solve_free_boundary``, ``turns`` (n_coils,) | None = config turns): ``currents`` (B, n_coils) CUDA float64
+        holds the starting currents in amperes and receives the final ones; ``w_dev`` is not used.  The result then
+        also has ``currents`` and ``shape_out`` (B, 2P+4): target, achieved flux, rmse, max |residual|, active bounds,
+        fallback flag of each equilibrium's last shape step."""
         params = self._picard_params()
-        B = int(w_dev.shape[0])
+        shape = bool(optimize_shape) and target_points is not None
+        B = int((currents if shape else w_dev).shape[0])
         ctx = self._context(B)
         pos = [(c["r"], c["z"]) for c in self.cfg["coils"]]
         nc = len(pos)
@@ -737,7 +770,13 @@ class BatchedFusionKernel(_GridMixin):
         ext = self.__dict__.get("_fb_ext")
         if ext is None or ext.shape[0] != B:
             ext = self._fb_ext = D.empty((B, self.NZ, self.NR), self.device)
-        if nc:
+        if shape:
+            tr = np.array([c.get("turns", 1) for c in self.cfg["coils"]], dtype=np.float64) if turns is None \
+                else np.asarray(turns, dtype=np.float64).reshape(-1)
+            spec = self._shape_spec(B, tr, target_points, target_values, current_limits, tikhonov_alpha)
+            if tuple(currents.shape) != (B, nc):
+                raise ValueError(f"currents must have shape ({B}, {nc}).")
+        elif nc:
             g = self._green_table(pos, 1)
             _lib.check(ctx.lib.gsb_coil_flux(ctx.handle, D.ptr(g), D.ptr(w_dev), nc, 1, D.ptr(ext), B, st), "gsb_coil_flux")
         else:
@@ -753,6 +792,9 @@ class BatchedFusionKernel(_GridMixin):
         fb = _lib.gsb_free_boundary_params()
         fb.max_outer_iter, fb.tol, fb.warm_j = int(max_outer_iter), float(tol), 0
         null = ctypes.c_void_p()
+        if shape:
+            return self._shape_solve_call(ctx, params, fb, spec, pos, currents, psi, ext, m, ip_dev, ped_dev, jphi, summ,
+                                          fbs, B, st, events)
         if events is not None:
             events[0].record()
         _lib.check(ctx.lib.gsb_free_boundary_solve(ctx.handle, ctypes.byref(params), ctypes.byref(fb), D.ptr(psi), D.ptr(ext),
@@ -762,6 +804,96 @@ class BatchedFusionKernel(_GridMixin):
         if events is not None:
             events[1].record()
         return {"psi": psi, "j_phi": jphi, "psi_ext": ext, "summary": summ, "fb_summary": fbs}
+
+    # -- shape-optimising outer loop --------------------------------------------------------------------
+    def _shape_spec(self, B: int, turns: np.ndarray, target_points, target_values, current_limits,
+                    tikhonov_alpha) -> dict[str, Any]:
+        """Check the shape-fit inputs with the reference's messages (free_boundary.py) and the device's limits."""
+        nc = len(self.cfg["coils"])
+        if nc == 0:
+            raise ValueError("CoilSet.positions must contain at least one coil.")
+        if nc > 32:
+            raise ValueError("optimize_shape supports at most 32 coils on the device.")
+        pts = np.ascontiguousarray(target_points, dtype=np.float64)
+        if pts.ndim != 2 or pts.shape[1] != 2 or pts.shape[0] == 0:
+            raise ValueError("target_flux_points must have shape (n_points, 2) with n_points > 0.")
+        if not np.all(np.isfinite(pts)):
+            raise ValueError("target_flux_points must contain finite values only.")
+        if np.any(pts[:, 0] <= 0.0):
+            raise ValueError("observation radii must be positive.")
+        P = pts.shape[0]
+        if P > 1024:
+            raise ValueError("optimize_shape supports at most 1024 target points on the device.")
+        vals = None
+        if target_values is not None:
+            v = np.asarray(target_values, dtype=np.float64)
+            if v.ndim == 1 and v.shape == (P,):
+                v = np.broadcast_to(v, (B, P))
+            elif v.shape != (B, P):
+                raise ValueError("target_flux_values must have the same length as target_flux_points.")
+            if not np.all(np.isfinite(v)):
+                raise ValueError("target_flux_values must contain finite values only.")
+            vals = np.ascontiguousarray(v)
+        alpha = float(tikhonov_alpha)
+        if not np.isfinite(alpha) or alpha < 0.0:
+            raise ValueError("tikhonov_alpha must be finite and non-negative.")
+        lim = None
+        if current_limits is not None:
+            lim = np.ascontiguousarray(current_limits, dtype=np.float64).reshape(-1)
+            if lim.shape[0] != nc:
+                raise ValueError("current_limits must have one entry per coil.")
+            if not np.all(np.isfinite(lim)):
+                raise ValueError("current_limits must contain finite values only.")
+            if np.any(lim <= 0.0):
+                raise ValueError("current_limits must contain finite positive values only.")
+        tr = np.asarray(turns, dtype=np.float64).reshape(-1)
+        if tr.shape[0] != nc or not np.all(np.isfinite(tr)) or np.any(tr < 1) or np.any(tr != np.round(tr)):
+            raise ValueError("turns must be positive integers when optimize_shape is set.")
+        return {"points": pts, "values": vals, "limits": lim, "alpha": alpha, "turns": tr.astype(np.int32)}
+
+    def _shape_solve_call(self, ctx, params, fb, spec, pos, currents, psi, ext, m, ip_dev, ped_dev, jphi, summ, fbs, B,
+                          st, events) -> dict[str, Any]:
+        dp = ctypes.POINTER(ctypes.c_double)
+        nc, P = len(pos), spec["points"].shape[0]
+        rz = np.ascontiguousarray(np.asarray(pos, dtype=np.float64).reshape(nc, 2))
+        sp = _lib.gsb_shape_params()
+        sp.n_coils, sp.coil_rz, sp.n_points = nc, rz.ctypes.data_as(dp), P
+        sp.points, sp.alpha = spec["points"].ctypes.data_as(dp), spec["alpha"]
+        sp.isoflux = 1 if spec["values"] is None else 0
+        sp.limits = spec["limits"].ctypes.data_as(dp) if spec["limits"] is not None else None
+        turns = spec["turns"]
+        tgt = None if spec["values"] is None else D.to_device(spec["values"], self.device)
+        out = D.empty((B, 2 * P + 4), self.device)
+        g = self._green_table(pos, 1)
+        null = ctypes.c_void_p()
+        if events is not None:
+            events[0].record()
+        _lib.check(ctx.lib.gsb_free_boundary_shape_solve(
+            ctx.handle, ctypes.byref(params), ctypes.byref(fb), ctypes.byref(sp), D.ptr(g),
+            turns.ctypes.data_as(ctypes.POINTER(ctypes.c_int)), D.ptr(currents), null if tgt is None else D.ptr(tgt),
+            D.ptr(out), D.ptr(psi), D.ptr(ext), null if m is None else D.ptr(m), D.ptr(ip_dev),
+            null if ped_dev is None else D.ptr(ped_dev), D.ptr(jphi), D.ptr(summ), D.ptr(fbs), B, st),
+            "gsb_free_boundary_shape_solve")
+        if events is not None:
+            events[1].record()
+        return {"psi": psi, "j_phi": jphi, "psi_ext": ext, "summary": summ, "fb_summary": fbs, "currents": currents,
+                "shape_out": out}
+
+    def _shape_report(self, spec, so: np.ndarray) -> dict[str, Any]:
+        """The reference's ``shape_optimization`` dict (fusion_kernel_free_boundary.py:686-699) over the batch."""
+        from .free_boundary import _mutual_device
+        pos = [(c["r"], c["z"]) for c in self.cfg["coils"]]
+        P = spec["points"].shape[0]
+        resp = _mutual_device(self.device, pos, spec["turns"], spec["points"])  # geometry only
+        tgt, ach = so[:, :P].copy(), so[:, P:2 * P].copy()
+        rmse = so[:, 2 * P].copy()
+        return {"solver_mode": "free_boundary_solver_shape_current_optimization", "target_point_count": int(P),
+                "coil_count": len(pos), "response_rank": int(np.linalg.matrix_rank(resp.T)),
+                "response_condition": float(np.linalg.cond(resp.T)), "flux_rmse": rmse,
+                "flux_relative_rmse": rmse / np.maximum(np.sqrt(np.mean(tgt ** 2, axis=1)), 1.0),
+                "max_abs_flux_residual": so[:, 2 * P + 1].copy(),
+                "active_current_bounds": so[:, 2 * P + 2].astype(np.int64), "target_flux": tgt,
+                "achieved_flux": ach, "fit_fallback": so[:, 2 * P + 3] > 0.5}
 
     def solve_device(self, w_dev, ip_dev, ped_dev=None, *, want_history: bool = False, psi_out=None,
                      jphi_out=None, events=None) -> dict[str, Any]:
