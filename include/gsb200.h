@@ -261,6 +261,34 @@ int gsb_free_boundary_shape_solve(gsb_ctx *ctx, const gsb_picard_params *p, cons
                                   const double *ip_dev, const double *prof_dev, double *jphi_dev, double *summary_dev,
                                   double *fb_summary_dev, int batch, void *stream);
 
+typedef struct gsb_probe_params {
+  int n_coils;             /* 1..32 */
+  int n_rows;              /* measurements m (flux loops, then B probes), 1..1024 */
+  const double *response;  /* HOST [m][n_coils] probe response R_p (build_magnetic_probe_response_matrix) */
+  const double *sigma;     /* HOST [m] measurement sigma (> 0; weights w = 1/sigma) or NULL (w = 1) */
+  double alpha;            /* Tikhonov weight (tikhonov_alpha), finite and >= 0 */
+  const double *limits;    /* HOST [n_coils] current limits (> 0; bounds are +-limits) or NULL (unbounded) */
+  int max_iter;            /* cap on the free-set solves of one fit; 0 = 3 n_coils + 10 */
+} gsb_probe_params;
+
+/* reconstruct_coil_currents_from_magnetic_probes (fusion_kernel_free_boundary.py:370-488) for `batch` independent
+ * measurement vectors of one diagnostic set.  Context-free: it runs on the current device and `stream`.  Each sample b
+ * gets the currents x minimising |diag(w) (R_p x - meas_b)|^2 + alpha |x - prior_b|^2 within +-limits: the exact
+ * minimiser (bounded-variable least squares on the QR factor of [diag(w) R_p; sqrt(alpha) I], factored once per
+ * call), where the reference stops lsq_linear(method="trf") at its tolerance.  With alpha = 0 the prior is not used.
+ * A rank-deficient factor (alpha = 0 and fewer independent rows than coils) fails with GSB_EINVAL before the fit.
+ * meas_dev      [batch][m] measurements (flux loops, then B probes)
+ * prior_dev     [batch][n_coils] prior currents
+ * currents_dev  [batch][n_coils] out: fitted currents (clip(prior, +-limits) where the fit failed)
+ * residual_dev  [batch][m] out: R_p x - meas;  wresidual_dev [batch][m] out: residual * w
+ * stats_dev     [batch][4] out: residual rms, weighted residual rms, active bounds (np.isclose(x, +-limit)),
+ *               failed (1: non-finite right-hand side or max_iter reached)
+ * work_dev      device workspace of *work_bytes bytes; with work_dev NULL the call only stores the size it needs in
+ *               *work_bytes (n_coils and n_rows must then be set). */
+int gsb_probe_reconstruct(const gsb_probe_params *pp, const double *meas_dev, const double *prior_dev,
+                          double *currents_dev, double *residual_dev, double *wresidual_dev, double *stats_dev,
+                          void *work_dev, long long *work_bytes, int batch, void *stream);
+
 /* Measurement hook (bench.py roofline): while enabled, gsb_free_boundary_solve brackets every inner Picard solve and
  * every wall GEMM with CUDA events on the launching stream and accumulates
  * out4 = {Picard solves: total ms, count; wall GEMMs: total ms, count}.  out4 may be NULL; reset != 0 zeroes the sums. */

@@ -41,6 +41,11 @@ class gsb_shape_params(ctypes.Structure):
                 ("alpha", c_double), ("isoflux", c_int), ("limits", POINTER(c_double))]
 
 
+class gsb_probe_params(ctypes.Structure):
+    _fields_ = [("n_coils", c_int), ("n_rows", c_int), ("response", POINTER(c_double)), ("sigma", POINTER(c_double)),
+                ("alpha", c_double), ("limits", POINTER(c_double)), ("max_iter", c_int)]
+
+
 _dp = POINTER(c_double)
 _ip = POINTER(c_int)
 
@@ -89,6 +94,8 @@ SIGNATURES = {
                                               POINTER(gsb_shape_params), c_void_p, _ip, c_void_p, c_void_p, c_void_p,
                                               c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                               c_void_p, c_int, c_void_p]),
+    "gsb_probe_reconstruct": (c_int, [POINTER(gsb_probe_params), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                      c_void_p, c_void_p, POINTER(c_longlong), c_int, c_void_p]),
     "gsb_enable_peer_access": (c_int, [c_int, c_int]),
     "gsb_ipc_alloc": (c_int, [c_int, c_longlong, POINTER(c_void_p), c_char_p]),
     "gsb_ipc_open": (c_int, [c_int, c_char_p, POINTER(c_void_p)]),

@@ -2063,9 +2063,90 @@ __device__ double shape_free_solve(const double *rs, double *ws, double *zs, int
   return z;
 }
 
-// One warp per active equilibrium, lane = coil: c = Q1^T t, then bounded-variable least squares (Stark & Parker 1995,
-// the algorithm of lsq_linear(method="bvls")) on min |R x - c| within [lo, hi]; then the fit diagnostics and the
-// coil weights x * turns.  A non-finite target or more than max_iter free-set solves keeps clip(prior, lo, hi).
+// Bounded-variable least squares (Stark & Parker 1995, the algorithm of lsq_linear(method="bvls")) on the n x n
+// problem min |R x - c| within [lo, hi], one warp, lane = coil (lanes >= n: coil = false).  rs = R [n][n] row-major;
+// ws [32*32] and zs [32] are the warp's scratch.  Writes this lane's x and returns false when more than max_iter
+// free-set solves would be needed (x is then unusable).  Called by whole warps only.
+__device__ __forceinline__ bool bvls_warp(const double *rs, double *ws, double *zs, int n, bool coil, double lo,
+                                          double hi, double c, int max_iter, double &x_out) {
+  const int lane = threadIdx.x & 31;
+  double cmax = coil ? fabs(c) : 0.0, rmax = 0.0;
+  for (int i = 0; i < n; ++i) rmax = fmax(rmax, coil ? fabs(rs[i * n + lane]) : 0.0);
+  cmax = warp_max(cmax);
+  rmax = warp_max(rmax);
+  bool fallback = false;
+  int bnd = 0;  // -1 at lo, +1 at hi, 0 free
+  double x = 0.0;
+  int iters = 0;
+  // start (as scipy's bvls): solve on the free set, put violators on their bounds, repeat until feasible
+  while (true) {
+    const bool fr = coil && bnd == 0;
+    if (!__any_sync(0xffffffffu, fr)) break;
+    const double z = shape_free_solve(rs, ws, zs, n, fr, c, x);
+    ++iters;
+    const bool below = fr && z < lo, above = fr && z > hi;
+    if (below) x = lo, bnd = -1;
+    if (above) x = hi, bnd = 1;
+    if (fr && !below && !above) x = z;
+    if (!__any_sync(0xffffffffu, below || above)) break;
+  }
+  bool excluded = false;  // just freed and pushed straight back out: not a candidate until the next free step
+  while (!fallback) {
+    // g = R^T (R x - c); lane = row for r, lane = column for g
+    double r = -c;
+    for (int j = 0; j < n; ++j) {
+      const double xj = __shfl_sync(0xffffffffu, x, j);
+      if (coil) r += rs[lane * n + j] * xj;
+    }
+    double gj = 0.0;
+    for (int i = 0; i < n; ++i) {
+      const double ri = __shfl_sync(0xffffffffu, r, i);
+      if (coil) gj += rs[i * n + lane] * ri;
+    }
+    const double xmax = warp_max(coil ? fabs(x) : 0.0);
+    const double thresh = 64.0 * n * 2.220446049250313e-16 * rmax * (rmax * xmax + cmax);
+    const double cand = (coil && bnd != 0 && !excluded) ? gj * (double)bnd : -INFINITY;
+    double best = warp_max(cand);
+    if (!(best > thresh)) break;  // KKT: no bound variable wants to move inwards
+    const int t = __ffs(__ballot_sync(0xffffffffu, cand == best)) - 1;
+    const int bnd_t = __shfl_sync(0xffffffffu, bnd, t);
+    if (lane == t) bnd = 0;
+    bool first = true;
+    while (true) {
+      if (++iters > max_iter) {
+        fallback = true;
+        break;
+      }
+      const bool fr = coil && bnd == 0;
+      const double z = shape_free_solve(rs, ws, zs, n, fr, c, x);
+      const bool below = fr && z < lo, above = fr && z > hi;
+      double step = (below || above) ? ((below ? lo : hi) - x) / (z - x) : INFINITY;
+      const double smin = warp_min_d(step);
+      if (smin == INFINITY) {
+        if (fr) x = z;
+        excluded = false;
+        break;
+      }
+      const int i = __ffs(__ballot_sync(0xffffffffu, step == smin)) - 1;
+      const int side_i = __shfl_sync(0xffffffffu, below ? -1 : 1, i);
+      // The freed variable leaves at once through the bound it came from: its inward gradient was rounding, so put
+      // it back and try the next candidate.  Leaving through the OPPOSITE bound is an ordinary step (it moves there).
+      if (first && i == t && side_i == bnd_t) {
+        if (lane == t) bnd = bnd_t, excluded = true;
+        break;
+      }
+      first = false;
+      if (fr) x = fmin(fmax(x + smin * (z - x), lo), hi);
+      if (lane == i) x = below ? lo : hi, bnd = below ? -1 : 1;
+    }
+  }
+  x_out = x;
+  return !fallback;
+}
+
+// One warp per active equilibrium, lane = coil: c = Q1^T t, then bvls_warp on min |R x - c| within [lo, hi]; then
+// the fit diagnostics and the coil weights x * turns.  A non-finite target or more than max_iter free-set solves keeps
+// clip(prior, lo, hi).
 __global__ void __launch_bounds__(32 * kShapeWarps) k_shape_fit(ShapeFitArgs g) {
   __shared__ double rs[kShapeMaxCoils * kShapeMaxCoils];
   __shared__ double ws_all[kShapeWarps][32 * 32];
@@ -2089,78 +2170,8 @@ __global__ void __launch_bounds__(32 * kShapeWarps) k_shape_fit(ShapeFitArgs g) 
     finite = finite && isfinite(t);
     if (coil) c += g.q1[(size_t)p * n + lane] * t;
   }
-  double cmax = coil ? fabs(c) : 0.0, rmax = 0.0;
-  for (int i = 0; i < n; ++i) rmax = fmax(rmax, coil ? fabs(rs[i * n + lane]) : 0.0);
-  cmax = warp_max(cmax);
-  rmax = warp_max(rmax);
-  bool fallback = !finite;
-  int bnd = 0;  // -1 at lo, +1 at hi, 0 free
   double x = 0.0;
-  int iters = 0;
-  if (!fallback) {
-    // start (as scipy's bvls): solve on the free set, put violators on their bounds, repeat until feasible
-    while (true) {
-      const bool fr = coil && bnd == 0;
-      if (!__any_sync(0xffffffffu, fr)) break;
-      const double z = shape_free_solve(rs, ws, zs, n, fr, c, x);
-      ++iters;
-      const bool below = fr && z < lo, above = fr && z > hi;
-      if (below) x = lo, bnd = -1;
-      if (above) x = hi, bnd = 1;
-      if (fr && !below && !above) x = z;
-      if (!__any_sync(0xffffffffu, below || above)) break;
-    }
-    bool excluded = false;  // just freed and pushed straight back out: not a candidate until the next free step
-    while (!fallback) {
-      // g = R^T (R x - c); lane = row for r, lane = column for g
-      double r = -c;
-      for (int j = 0; j < n; ++j) {
-        const double xj = __shfl_sync(0xffffffffu, x, j);
-        if (coil) r += rs[lane * n + j] * xj;
-      }
-      double gj = 0.0;
-      for (int i = 0; i < n; ++i) {
-        const double ri = __shfl_sync(0xffffffffu, r, i);
-        if (coil) gj += rs[i * n + lane] * ri;
-      }
-      const double xmax = warp_max(coil ? fabs(x) : 0.0);
-      const double thresh = 64.0 * n * 2.220446049250313e-16 * rmax * (rmax * xmax + cmax);
-      const double cand = (coil && bnd != 0 && !excluded) ? gj * (double)bnd : -INFINITY;
-      double best = warp_max(cand);
-      if (!(best > thresh)) break;  // KKT: no bound variable wants to move inwards
-      const int t = __ffs(__ballot_sync(0xffffffffu, cand == best)) - 1;
-      const int bnd_t = __shfl_sync(0xffffffffu, bnd, t);
-      if (lane == t) bnd = 0;
-      bool first = true;
-      while (true) {
-        if (++iters > g.max_iter) {
-          fallback = true;
-          break;
-        }
-        const bool fr = coil && bnd == 0;
-        const double z = shape_free_solve(rs, ws, zs, n, fr, c, x);
-        const bool below = fr && z < lo, above = fr && z > hi;
-        double step = (below || above) ? ((below ? lo : hi) - x) / (z - x) : INFINITY;
-        const double smin = warp_min_d(step);
-        if (smin == INFINITY) {
-          if (fr) x = z;
-          excluded = false;
-          break;
-        }
-        const int i = __ffs(__ballot_sync(0xffffffffu, step == smin)) - 1;
-        const int side_i = __shfl_sync(0xffffffffu, below ? -1 : 1, i);
-        // The freed variable leaves at once through the bound it came from: its inward gradient was rounding, so put
-        // it back and try the next candidate.  Leaving through the OPPOSITE bound is an ordinary step (it moves there).
-        if (first && i == t && side_i == bnd_t) {
-          if (lane == t) bnd = bnd_t, excluded = true;
-          break;
-        }
-        first = false;
-        if (fr) x = fmin(fmax(x + smin * (z - x), lo), hi);
-        if (lane == i) x = below ? lo : hi, bnd = below ? -1 : 1;
-      }
-    }
-  }
+  const bool fallback = !finite || !bvls_warp(rs, ws, zs, n, coil, lo, hi, c, g.max_iter, x);
   if (fallback) x = fmin(fmax(prior, lo), hi);
   if (!coil) x = 0.0;
   zs[lane] = x;
@@ -2198,6 +2209,97 @@ __global__ void k_shape_weights(const double *__restrict__ cur, const double *__
                                 double *__restrict__ w) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < total) w[i] = dmul(cur[i], turns[i % n]);
+}
+
+// ---------------------------------------------------------------------------- magnetic-probe current reconstruction
+// (reconstruct_coil_currents_from_magnetic_probes, fusion_kernel_free_boundary.py:370-488).  A = [diag(w) R_p;
+// sqrt(alpha) I] is geometry only, so k_shape_factor factors it once per call (its M^T is diag(w) R_p) and every sample
+// solves min |R x - c| with c = Q1^T (w o meas) + Q2^T (sqrt(alpha) prior), whose minimiser is that of
+// |A x - [w o meas; sqrt(alpha) prior]|.
+struct ProbeFitArgs {
+  const double *rmat;    // [n][n]
+  const double *q1;      // [m][n]
+  const double *q;       // Q of k_shape_factor, column-major [(m+n)][n]: rows m..m+n-1 are Q2
+  const double *resp_t;  // [n][m] unweighted response, transposed
+  const double *w;       // [m] 1/sigma
+  const double *lim;     // [n] or NULL
+  const double *meas;    // [B][m]
+  const double *prior;   // [B][n]
+  double *currents;      // [B][n]
+  double *residual;      // [B][m] R_p x - meas
+  double *wresidual;     // [B][m] residual * w
+  double *stats;         // [B][4] residual_rms, weighted_residual_rms, active bounds, failed
+  double sqrt_alpha;
+  int n, m, batch, max_iter;
+};
+
+// One warp per sample, lane = coil.  A non-finite right-hand side or more than max_iter free-set solves sets the
+// failure flag and leaves clip(prior, lo, hi) as the currents.
+__global__ void __launch_bounds__(32 * kShapeWarps) k_probe_fit(ProbeFitArgs g) {
+  __shared__ double rs[kShapeMaxCoils * kShapeMaxCoils];
+  __shared__ double ws_all[kShapeWarps][32 * 32];
+  __shared__ double zs_all[kShapeWarps][32];
+  const int n = g.n, m = g.m;
+  for (int i = threadIdx.x; i < n * n; i += blockDim.x) rs[i] = g.rmat[i];
+  __syncthreads();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int b = blockIdx.x * kShapeWarps + warp;
+  if (b >= g.batch) return;
+  double *ws = ws_all[warp], *zs = zs_all[warp];
+  const double *mb = g.meas + (size_t)b * m;
+  const bool coil = lane < n;
+  const double lim = (coil && g.lim) ? g.lim[lane] : INFINITY;
+  const double lo = -lim, hi = lim;
+  const double prior = coil ? g.prior[(size_t)b * n + lane] : 0.0;
+  // c = Q1^T (w o meas) + Q2^T (sqrt(alpha) prior), rows in order; the measurement rows arrive 32 at a time
+  double c = 0.0;
+  for (int i0 = 0; i0 < m; i0 += 32) {
+    const double v = i0 + lane < m ? dmul(mb[i0 + lane], g.w[i0 + lane]) : 0.0;
+    const int cnt = min(32, m - i0);
+    for (int r = 0; r < cnt; ++r) {
+      const double t = __shfl_sync(0xffffffffu, v, r);
+      if (coil) c += g.q1[(size_t)(i0 + r) * n + lane] * t;
+    }
+  }
+  if (g.sqrt_alpha > 0.0) {  // alpha = 0: the reference drops the prior rows
+    const double v = dmul(g.sqrt_alpha, prior);
+    const double *q2 = g.q + (size_t)lane * (m + n) + m;
+    for (int k = 0; k < n; ++k) {
+      const double t = __shfl_sync(0xffffffffu, v, k);
+      if (coil) c += q2[k] * t;
+    }
+  }
+  const bool finite = __all_sync(0xffffffffu, !coil || isfinite(c));
+  double x = 0.0;
+  const bool failed = !finite || !bvls_warp(rs, ws, zs, n, coil, lo, hi, c, g.max_iter, x);
+  if (failed) x = fmin(fmax(prior, lo), hi);
+  if (!coil) x = 0.0;
+  zs[lane] = x;
+  __syncwarp();
+  if (coil) g.currents[(size_t)b * n + lane] = x;
+  double ss = 0.0, wss = 0.0;
+  for (int i = lane; i < m; i += 32) {
+    double a = 0.0;
+    for (int j = 0; j < n; ++j) a += g.resp_t[(size_t)j * m + i] * zs[j];
+    const double r = a - mb[i], wr = dmul(r, g.w[i]);
+    g.residual[(size_t)b * m + i] = r;
+    g.wresidual[(size_t)b * m + i] = wr;
+    ss += r * r;
+    wss += wr * wr;
+  }
+  ss = warp_sum(ss);
+  wss = warp_sum(wss);
+  // np.isclose(x, lb) | np.isclose(x, ub): |x - b| <= 1e-8 + 1e-5 |b|, never true for an infinite bound
+  const double tol = 1e-8 + 1e-5 * lim;
+  const int active =
+      __popc(__ballot_sync(0xffffffffu, coil && g.lim && (fabs(x - lo) <= tol || fabs(x - hi) <= tol)));
+  if (lane == 0) {
+    double *s = g.stats + (size_t)b * 4;
+    s[0] = sqrt(ss / (double)m);
+    s[1] = sqrt(wss / (double)m);
+    s[2] = (double)active;
+    s[3] = failed ? 1.0 : 0.0;
+  }
 }
 
 }  // namespace gsb
@@ -3006,6 +3108,87 @@ int gsb_free_boundary_shape_solve(gsb_ctx *ctx, const gsb_picard_params *p, cons
   sh.green = green_dev;
   return free_boundary_loop(ctx, p, fb, &sh, psi_dev, psi_ext_dev, wall_m_dev, ip_dev, prof_dev, jphi_dev,
                             summary_dev, fb_summary_dev, batch, stream);
+}
+
+int gsb_probe_reconstruct(const gsb_probe_params *pp, const double *meas_dev, const double *prior_dev,
+                          double *currents_dev, double *residual_dev, double *wresidual_dev, double *stats_dev,
+                          void *work_dev, long long *work_bytes, int batch, void *stream) {
+  // every argument is checked here, before the first launch
+  GSB_REQUIRE(pp && work_bytes, "gsb_probe_reconstruct: NULL argument");
+  const int n = pp->n_coils, m = pp->n_rows;
+  GSB_REQUIRE(n >= 1 && n <= kShapeMaxCoils, "probe reconstruction supports 1 to 32 coils on the device.");
+  GSB_REQUIRE(m >= 1 && m <= kShapeMaxPoints, "probe reconstruction supports 1 to 1024 measurements on the device.");
+  // workspace: host block {diag(w) R_p transposed [n][m] | R_p transposed [n][m] | w [m] | limits [n]} | A, Q
+  // [(m+n)][n] | R [n][n] | Q1 [m][n] | rank flag
+  const size_t mn = (size_t)m * n, host_n = 2 * mn + m + n, nd = host_n + 2 * (mn + (size_t)n * n) + (size_t)n * n + mn;
+  const size_t need = nd * sizeof(double) + sizeof(int);
+  if (!work_dev) {
+    *work_bytes = (long long)need;
+    return GSB_OK;
+  }
+  GSB_REQUIRE(*work_bytes >= (long long)need, "gsb_probe_reconstruct: workspace too small");
+  GSB_REQUIRE(meas_dev && prior_dev && currents_dev && residual_dev && wresidual_dev && stats_dev && pp->response,
+              "gsb_probe_reconstruct: NULL argument");
+  GSB_REQUIRE(batch >= 1, "gsb_probe_reconstruct: batch must be >= 1");
+  GSB_REQUIRE(pp->max_iter >= 0, "gsb_probe_reconstruct: max_iter must be >= 0");
+  GSB_REQUIRE(std::isfinite(pp->alpha) && pp->alpha >= 0.0, "tikhonov_alpha must be finite and non-negative.");
+  for (size_t k = 0; k < mn; ++k)
+    GSB_REQUIRE(std::isfinite(pp->response[k]), "Magnetic probe response matrix contains non-finite entries.");
+  if (pp->sigma)
+    for (int i = 0; i < m; ++i)
+      GSB_REQUIRE(std::isfinite(pp->sigma[i]) && pp->sigma[i] > 0.0,
+                  "measurement_sigma must contain finite positive values only.");
+  if (pp->limits)
+    for (int j = 0; j < n; ++j)
+      GSB_REQUIRE(std::isfinite(pp->limits[j]) && pp->limits[j] > 0.0,
+                  "current_limits must contain finite positive values only.");
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<double> host(host_n);
+  double *h_a = host.data(), *h_r = h_a + mn, *h_w = h_r + mn, *h_lim = h_w + m;
+  for (int i = 0; i < m; ++i) {
+    const double w = pp->sigma ? 1.0 / pp->sigma[i] : 1.0;
+    h_w[i] = w;
+    for (int j = 0; j < n; ++j) {
+      const double r = pp->response[(size_t)i * n + j];
+      h_a[(size_t)j * m + i] = r * w;  // resp * w[:, None]
+      h_r[(size_t)j * m + i] = r;
+    }
+  }
+  for (int j = 0; j < n; ++j) h_lim[j] = pp->limits ? pp->limits[j] : 0.0;
+  double *d_host = (double *)work_dev, *d_a = d_host + host_n, *d_q = d_a + (mn + (size_t)n * n),
+         *d_r = d_q + (mn + (size_t)n * n), *d_q1 = d_r + (size_t)n * n;
+  int *d_flag = (int *)(d_host + nd);
+  GSB_CUDA(cudaMemcpyAsync(d_host, host.data(), host.size() * sizeof(double), cudaMemcpyHostToDevice, st));
+  const double sqrt_alpha = std::sqrt(pp->alpha);
+  k_shape_factor<<<1, 1024, 0, st>>>(d_host, n, m, sqrt_alpha, d_a, d_q, d_r, d_q1, d_flag);
+  GSB_LAUNCH_CHECK();
+  int deficient = 0;
+  GSB_CUDA(cudaMemcpyAsync(&deficient, d_flag, sizeof(int), cudaMemcpyDeviceToHost, st));
+  GSB_CUDA(cudaStreamSynchronize(st));
+  GSB_REQUIRE(deficient == 0,
+              "the probe fit [diag(w) R; sqrt(tikhonov_alpha) I] is rank deficient: use tikhonov_alpha > 0 or more "
+              "independent measurements");
+  ProbeFitArgs a{};
+  a.rmat = d_r;
+  a.q1 = d_q1;
+  a.q = d_q;
+  a.resp_t = d_host + mn;
+  a.w = d_host + 2 * mn;
+  a.lim = pp->limits ? d_host + 2 * mn + m : nullptr;
+  a.meas = meas_dev;
+  a.prior = prior_dev;
+  a.currents = currents_dev;
+  a.residual = residual_dev;
+  a.wresidual = wresidual_dev;
+  a.stats = stats_dev;
+  a.sqrt_alpha = sqrt_alpha;
+  a.n = n;
+  a.m = m;
+  a.batch = batch;
+  a.max_iter = pp->max_iter > 0 ? pp->max_iter : 3 * n + 10;
+  k_probe_fit<<<(batch + kShapeWarps - 1) / kShapeWarps, 32 * kShapeWarps, 0, st>>>(a);
+  GSB_LAUNCH_CHECK();
+  return GSB_OK;
 }
 
 int gsb_timing(gsb_ctx *ctx, int enable, double *out4, int reset) {

@@ -117,6 +117,18 @@ def validate_config(raw: dict[str, Any]) -> dict[str, Any]:
     return cfg
 
 
+def _measurement_rows(value, name: str, length: int) -> np.ndarray:
+    """(B, length) float64 rows of a batched measurement argument; a 1-D vector is a batch of one."""
+    a = np.asarray(value, dtype=np.float64)
+    if a.ndim == 1:
+        a = a[None, :]
+    if a.ndim != 2 or a.shape[1] != length or a.shape[0] < 1:
+        raise ValueError(f"{name} must have length {length}.")
+    if not np.all(np.isfinite(a)):
+        raise ValueError(f"{name} must contain finite values only.")
+    return a
+
+
 def _load_config(src) -> dict[str, Any]:
     if isinstance(src, dict):
         return validate_config(src)
@@ -894,6 +906,127 @@ class BatchedFusionKernel(_GridMixin):
                 "max_abs_flux_residual": so[:, 2 * P + 1].copy(),
                 "active_current_bounds": so[:, 2 * P + 2].astype(np.int64), "target_flux": tgt,
                 "achieved_flux": ach, "fit_fallback": so[:, 2 * P + 3] > 0.5}
+
+    # -- magnetic-probe current reconstruction -----------------------------------------------------------
+    def reconstruct_coil_currents_from_magnetic_probes(self, *, flux_points=None, flux_measurements=None,
+                                                       b_probe_points=None, b_probe_directions=None,
+                                                       b_probe_measurements=None, measurement_sigma=None,
+                                                       tikhonov_alpha: float = 1.0e-6, coil_currents=None,
+                                                       current_limits=None, turns=None) -> dict[str, Any]:
+        """``FusionKernel.reconstruct_coil_currents_from_magnetic_probes`` (fusion_kernel_free_boundary.py:370-488) for
+        B measurement vectors of one diagnostic set, fitted on the device in one call (gsb_probe_reconstruct).
+
+        flux_measurements (B, n_flux) and b_probe_measurements (B, n_b) (a 1-D vector is a batch of one) follow the
+        rows of ``build_magnetic_probe_response_matrix``; coil_currents (B, n_coils) | (n_coils,) | None (config
+        currents) is the prior of the Tikhonov term; measurement_sigma (m,) and current_limits (n_coils,) are shared
+        by the batch; turns (n_coils,) | None = config turns.  Each sample gets the exact bounded minimiser of
+        |w (R x - meas)|^2 + alpha |x - prior|^2 within +-current_limits, where the reference stops
+        ``lsq_linear(method="trf")`` at its tolerance (a current trf leaves just inside its limit sits on it here).
+        Returns the reference's keys with a leading batch axis where the value is per sample: coil_currents (B, n),
+        residual / weighted_residual (B, m), residual_rms / weighted_residual_rms / active_bounds (B,); response_rank
+        and response_condition of the unweighted response.  Raises ``RuntimeError`` naming the samples whose fit
+        failed (non-finite right-hand side or iteration cap), as the reference raises for its one sample.
+        """
+        from .free_boundary import _bounds, _points, _vector, build_magnetic_probe_response_matrix
+        cfg_coils = self.cfg["coils"]
+        n = len(cfg_coils)
+        if n > 32:
+            raise ValueError("probe reconstruction supports at most 32 coils on the device.")
+        tr = np.array([c.get("turns", 1) for c in cfg_coils], dtype=np.float64) if turns is None \
+            else np.asarray(turns, dtype=np.float64).reshape(-1)
+        if tr.shape[0] != n or not np.all(np.isfinite(tr)) or np.any(tr < 1) or np.any(tr != np.round(tr)):
+            raise ValueError("turns must be positive integers.")
+        coils = CoilSet(positions=[(c["r"], c["z"]) for c in cfg_coils],
+                        currents=np.array([c.get("current", 0.0) for c in cfg_coils], dtype=np.float64),
+                        turns=[int(t) for t in tr], current_limits=current_limits)
+        resp = build_magnetic_probe_response_matrix(self, coils, flux_points=flux_points, b_probe_points=b_probe_points,
+                                                    b_probe_directions=b_probe_directions)
+        parts = []
+        for pts, vals, pname, vname in ((flux_points, flux_measurements, "flux_points", "flux_measurements"),
+                                        (b_probe_points, b_probe_measurements, "b_probe_points", "b_probe_measurements")):
+            if pts is not None:
+                if vals is None:
+                    raise ValueError(f"{vname} must be provided with {pname}.")
+                parts.append(_measurement_rows(vals, vname, _points(pts, pname).shape[0]))
+            elif vals is not None:
+                raise ValueError(f"{pname} must be provided with {vname}.")
+        if not parts:
+            raise ValueError("At least one measurement vector must be provided.")
+        if len({p.shape[0] for p in parts}) > 1:
+            raise ValueError("flux_measurements and b_probe_measurements must have the same batch size.")
+        meas = np.ascontiguousarray(np.concatenate(parts, axis=1))
+        B, m = meas.shape
+        if m != resp.shape[0]:
+            raise ValueError("measurement vector length must match response rows.")
+        if m > 1024:
+            raise ValueError("probe reconstruction supports at most 1024 measurements on the device.")
+        sg = None
+        if measurement_sigma is not None:
+            sg = _vector(measurement_sigma, "measurement_sigma", m)
+            if np.any(sg <= 0.0):
+                raise ValueError("measurement_sigma must contain finite positive values only.")
+        alpha = float(tikhonov_alpha)
+        if not np.isfinite(alpha) or alpha < 0.0:
+            raise ValueError("tikhonov_alpha must be finite and non-negative.")
+        prior = coils.currents if coil_currents is None else np.asarray(coil_currents, dtype=np.float64)
+        if prior.ndim == 1 and prior.shape == (n,):
+            prior = np.tile(prior, (B, 1))
+        if prior.shape != (B, n) or not np.all(np.isfinite(prior)):
+            raise ValueError("CoilSet.currents must be finite with one entry per coil.")
+        lim = None if current_limits is None else _bounds(coils, n, positive=True)[1]
+        dev = self.reconstruct_coil_currents_device(resp, D.to_device(meas, self.device),
+                                                    D.to_device(prior, self.device), measurement_sigma=sg,
+                                                    tikhonov_alpha=alpha, current_limits=lim)
+        stats = dev["stats"].cpu().numpy()
+        bad = np.flatnonzero(stats[:, 3] > 0.5)
+        if bad.size:
+            raise RuntimeError("Magnetic probe inverse reconstruction failed: non-finite right-hand side or iteration "
+                               f"cap reached in samples {bad.tolist()}")
+        return {"coil_currents": dev["currents"].cpu().numpy(), "residual": dev["residual"].cpu().numpy(),
+                "weighted_residual": dev["weighted_residual"].cpu().numpy(), "residual_rms": stats[:, 0].copy(),
+                "weighted_residual_rms": stats[:, 1].copy(), "response_rank": int(np.linalg.matrix_rank(resp)),
+                "response_condition": float(np.linalg.cond(resp)), "active_bounds": stats[:, 2].astype(np.int64)}
+
+    def reconstruct_coil_currents_device(self, response, meas_dev, prior_dev, *, measurement_sigma=None,
+                                         tikhonov_alpha: float = 1.0e-6, current_limits=None, max_iter: int = 0,
+                                         events=None) -> dict[str, Any]:
+        """Device-resident probe fit (gsb_probe_reconstruct): response (m, n_coils) host array, meas_dev (B, m) and
+        prior_dev (B, n_coils) CUDA float64 tensors, measurement_sigma (m,) | None, current_limits (n_coils,) | None
+        (positive), max_iter = cap on the free-set solves per fit (0: 3 n_coils + 10).  Returns device tensors
+        currents (B, n), residual, weighted_residual (B, m) and stats (B, 4): residual rms, weighted residual rms,
+        active bounds, failed."""
+        lib = _lib.load()
+        dp = ctypes.POINTER(ctypes.c_double)
+        resp = np.ascontiguousarray(response, dtype=np.float64)
+        m, n = resp.shape
+        B = int(meas_dev.shape[0])
+        torch = D.torch_mod()
+        for t, shape, name in ((meas_dev, (B, m), "meas_dev"), (prior_dev, (B, n), "prior_dev")):
+            if tuple(t.shape) != shape or t.dtype != torch.float64 or not t.is_contiguous() or not t.is_cuda:
+                raise ValueError(f"{name} must be a contiguous CUDA float64 tensor of shape {shape}.")
+        sg = None if measurement_sigma is None else np.ascontiguousarray(measurement_sigma, dtype=np.float64)
+        lim = None if current_limits is None else np.ascontiguousarray(current_limits, dtype=np.float64)
+        pp = _lib.gsb_probe_params()
+        pp.n_coils, pp.n_rows, pp.response = n, m, resp.ctypes.data_as(dp)
+        pp.sigma = None if sg is None else sg.ctypes.data_as(dp)
+        pp.alpha, pp.max_iter = float(tikhonov_alpha), int(max_iter)
+        pp.limits = None if lim is None else lim.ctypes.data_as(dp)
+        null = ctypes.c_void_p()
+        need = ctypes.c_longlong(0)
+        _lib.check(lib.gsb_probe_reconstruct(ctypes.byref(pp), null, null, null, null, null, null, null,
+                                             ctypes.byref(need), B, null), "gsb_probe_reconstruct")
+        work = D.empty(((need.value + 7) // 8,), self.device)
+        need.value = work.numel() * 8
+        cur, stats = D.empty((B, n), self.device), D.empty((B, 4), self.device)
+        res, wres = D.empty((B, m), self.device), D.empty((B, m), self.device)
+        if events is not None:
+            events[0].record()
+        _lib.check(lib.gsb_probe_reconstruct(ctypes.byref(pp), D.ptr(meas_dev), D.ptr(prior_dev), D.ptr(cur), D.ptr(res),
+                                             D.ptr(wres), D.ptr(stats), D.ptr(work), ctypes.byref(need), B,
+                                             D.stream_ptr()), "gsb_probe_reconstruct")
+        if events is not None:
+            events[1].record()
+        return {"currents": cur, "residual": res, "weighted_residual": wres, "stats": stats}
 
     def solve_device(self, w_dev, ip_dev, ped_dev=None, *, want_history: bool = False, psi_out=None,
                      jphi_out=None, events=None) -> dict[str, Any]:
