@@ -150,17 +150,14 @@ int ensure_plan(gsb_ctx *ctx, int min_grid) {
     ctx->levels.push_back(D);
   }
   ctx->planned_min_grid = min_grid;
-  // first level from which the whole V-cycle tail fits one SM's shared memory
-  const char *env = getenv("GSB_NO_RESIDENT");
+  // first level from which the whole V-cycle tail fits one SM's shared memory (none: res_l0 = level count)
   ctx->res_l0 = (int)ctx->levels.size();
-  if (!(env && env[0] == '1')) {
-    RPlan plan;
-    for (int l0 = 0; l0 < (int)ctx->levels.size(); ++l0)
-      if (build_rplan(ctx, l0, 0, &plan)) {
-        ctx->res_l0 = l0;
-        break;
-      }
-  }
+  RPlan plan;
+  for (int l0 = 0; l0 < (int)ctx->levels.size(); ++l0)
+    if (build_rplan(ctx, l0, 0, &plan)) {
+      ctx->res_l0 = l0;
+      break;
+    }
   if (ctx->res_l0 == 0 && !ctx->split_src) {
     const size_t hw = (ctx->nr + 1) / 2;
     GSB_CUDA(cudaMalloc(&ctx->split_src, (size_t)ctx->batch_cap * 2 * ctx->nz * hw * sizeof(double)));

@@ -191,21 +191,21 @@ k_wall_matrix(const double *__restrict__ rrow, const double *__restrict__ zax, i
 //     loads (row = lane/4, k = lane%4) and the 8-byte cp.async fills (16 consecutive k per row) are both
 //     bank-conflict free;
 //   * 4-stage cp.async pipeline (zero-fill for the ragged last chunk of every grid row and for rows beyond
-//     the batch / the wall), one barrier per K tile;
+//     the batch / the wall) with full / empty mbarriers per stage instead of a CTA barrier per K tile
+//     (the alternatives measured against this configuration: profiles/r2_wall_gemm.md);
 //   * the interior gather is fused into the X-tile addressing: K is walked as (interior row, 16-column
 //     chunk), so a K tile never straddles a grid row and needs no per-element index arithmetic; dA is
 //     applied to the accumulators.
 // ------------------------------------------------------------------------------------------
 // Tile configuration: BM(b) x BN(w) x BK, NST cp.async stages, (BM/32) x (BN/32) warps of 32x32, CPS CTAs per SM.
-template <int BM_, int BN_, int BK_, int NST_, int CPS_, bool MBAR_ = false>
+template <int BM_, int BN_, int BK_, int NST_, int CPS_>
 struct GemmCfg {
   static constexpr int BM = BM_, BN = BN_, BK = BK_, NST = NST_, CPS = CPS_;
-  static constexpr bool MBAR = MBAR_;  // mbarrier full/empty pipeline instead of one __syncthreads per K tile
   static constexpr int LD = BK + 4;  // row pitch in doubles: (4*row + k) mod 16 distinct over a half warp -> no bank conflicts
   static constexpr int THREADS = (BM / 32) * (BN / 32) * 32;
   static constexpr int WN = BN / 32;  // warps along w
   static constexpr int STAGE = (BM + BN) * LD;
-  static constexpr int SMEM = NST * STAGE * (int)sizeof(double) + (MBAR_ ? 2 * NST * 8 : 0);
+  static constexpr int SMEM = NST * STAGE * (int)sizeof(double) + 2 * NST * 8;  // + full / empty mbarriers
   static constexpr int RP = THREADS / BK;  // rows filled per loader pass
 };
 
@@ -214,14 +214,6 @@ __device__ __forceinline__ void dmma884(double &c0, double &c1, double a, double
                : "+d"(c0), "+d"(c1)
                : "d"(a), "d"(b));
 }
-__device__ __forceinline__ void cp_async8(double *smem_dst, const double *gsrc, bool valid) {
-  const unsigned d = (unsigned)__cvta_generic_to_shared(smem_dst);
-  const int sz = valid ? 8 : 0;  // src-size 0: the 8 destination bytes are zero-filled
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(d), "l"(gsrc), "r"(sz) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 // mbarrier helpers (shared::cta, 32-bit shared addresses)
 __device__ __forceinline__ void mbar_init(unsigned bar, int count) {
   asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count) : "memory");
@@ -276,11 +268,9 @@ __global__ void __launch_bounds__(C::THREADS, C::CPS) k_wall_gemm_sk(const WallG
   // read it, so warps may drift apart by up to a tile instead of meeting at a CTA barrier every K tile.
   const unsigned bar_full = (unsigned)__cvta_generic_to_shared(gsm + NST * C::STAGE), bar_empty = bar_full + NST * 8;
   unsigned it = 0;  // K tiles consumed by this CTA so far (stage = it % NST, phase parity = (it / NST) & 1)
-  if (C::MBAR) {
-    if (tid == 0)
-      for (int st = 0; st < NST; ++st) mbar_init(bar_full + 8 * st, C::THREADS), mbar_init(bar_empty + 8 * st, C::THREADS / 32);
-    __syncthreads();
-  }
+  if (tid == 0)
+    for (int st = 0; st < NST; ++st) mbar_init(bar_full + 8 * st, C::THREADS), mbar_init(bar_empty + 8 * st, C::THREADS / 32);
+  __syncthreads();
   while (s < s_end) {
     const int tile = (int)(s / a.ntk), k_lo = (int)(s - (long long)tile * a.ntk);
     const int k_hi = (int)min((long long)a.ntk, k_lo + (s_end - s));
@@ -329,30 +319,13 @@ __global__ void __launch_bounds__(C::THREADS, C::CPS) k_wall_gemm_sk(const WallG
       issue((int)sj);
       mbar_arrive_on_cp_async(bar_full + 8 * sj);
     };
-    if (C::MBAR) {
 #pragma unroll
-      for (int st = 0; st < NST - 2; ++st)
-        if (st < nk) produce(it + st);
-    } else {
-#pragma unroll
-      for (int st = 0; st < NST - 1; ++st) {
-        if (st < nk) issue(st);
-        cp_async_commit();
-      }
-    }
+    for (int st = 0; st < NST - 2; ++st)
+      if (st < nk) produce(it + st);
     for (int i = 0; i < nk; ++i) {
-      int stage;
-      if (C::MBAR) {
-        stage = (int)((it + i) % NST);
-        if (i + NST - 2 < nk) produce(it + i + NST - 2);
-        mbar_wait(bar_full + 8 * stage, ((it + i) / NST) & 1);
-      } else {
-        stage = i % NST;
-        cp_async_wait<NST - 2>();
-        __syncthreads();  // tile i has landed for everybody; everybody is done reading the stage refilled next
-        if (i + NST - 1 < nk) issue((i + NST - 1) % NST);
-        cp_async_commit();
-      }
+      const int stage = (int)((it + i) % NST);
+      if (i + NST - 2 < nk) produce(it + i + NST - 2);
+      mbar_wait(bar_full + 8 * stage, ((it + i) / NST) & 1);
       const double *sX = gsm + stage * C::STAGE, *sM = sX + BM * LD;
 #pragma unroll
       for (int ks = 0; ks < BK; ks += 4) {
@@ -366,17 +339,10 @@ __global__ void __launch_bounds__(C::THREADS, C::CPS) k_wall_gemm_sk(const WallG
 #pragma unroll
           for (int v = 0; v < 4; ++v) dmma884(acc[u][v][0], acc[u][v][1], af[u], bf[v]);
       }
-      if (C::MBAR) {
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_empty + 8 * stage);
-      }
+      __syncwarp();
+      if (lane == 0) mbar_arrive(bar_empty + 8 * stage);
     }
-    if (C::MBAR) {
-      it += nk;
-    } else {
-      cp_async_wait<0>();
-      __syncthreads();  // the stages are refilled by the next segment
-    }
+    it += nk;
     // C fragment: row = gid, cols = 2*tig, 2*tig + 1
     const bool whole = (k_lo == 0 && k_hi == a.ntk);
     if (whole) {
@@ -560,16 +526,8 @@ int gsb_wall_flux(gsb_ctx *ctx, const double *m_dev, const double *jphi_dev, dou
   a.out = wall_dev;
   a.nz = ctx->nz, a.nr = ctx->nr, a.batch = batch, a.nwall = ctx->n_wall, a.nint = ctx->n_int;
   a.dA = dA;
-  // Tile configuration.  Default: 128x128x16 tiles, 4 stages, mbarrier full/empty pipeline, one CTA per SM.
-  // GSB_GEMM_VARIANT selects the measured alternatives (profiles/r2_wall_gemm.md): 1 = the same tiles with a
-  // __syncthreads() per K tile, 2 = 128x64 tiles, two CTAs per SM, mbarrier pipeline, 3 = three stages.
-  const char *env = getenv("GSB_GEMM_VARIANT");
-  switch (env ? atoi(env) : 0) {
-    case 1: return wall_gemm_launch<GemmCfg<128, 128, 16, 4, 1, false>>(ctx, a, st);
-    case 2: return wall_gemm_launch<GemmCfg<128, 64, 16, 3, 2, true>>(ctx, a, st);
-    case 3: return wall_gemm_launch<GemmCfg<128, 128, 16, 3, 1, true>>(ctx, a, st);
-    default: return wall_gemm_launch<GemmCfg<128, 128, 16, 4, 1, true>>(ctx, a, st);
-  }
+  // 128x128x16 tiles, 4 stages, one CTA per SM: the fastest of the configurations in profiles/r2_wall_gemm.md
+  return wall_gemm_launch<GemmCfg<128, 128, 16, 4, 1>>(ctx, a, st);
 }
 
 int gsb_wall_scatter(gsb_ctx *ctx, const double *wall_dev, double *bc_dev, int accumulate, int batch, void *stream) {

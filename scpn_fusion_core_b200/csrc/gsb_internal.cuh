@@ -75,28 +75,15 @@ constexpr int kMaxDevices = 64;
   } while (0)
 
 // ---------------------------------------------------------------- exact FP64 helpers
-#ifdef GSB_FMA
-// Experimental build (make fma -> libgsb200_fma.so, never the shipped library): plain operators, so nvcc contracts
-// a*b+c into DFMA, and divisions by precomputed constants become one multiplication by the reciprocal.  Results
-// are no longer bit-identical to NumPy; used to MEASURE what the exactness contract costs (profiles/).
-__device__ __forceinline__ double dmul(double a, double b) { return a * b; }
-__device__ __forceinline__ double dadd(double a, double b) { return a + b; }
-__device__ __forceinline__ double dsub(double a, double b) { return a - b; }
-#else
 __device__ __forceinline__ double dmul(double a, double b) { return __dmul_rn(a, b); }
 __device__ __forceinline__ double dadd(double a, double b) { return __dadd_rn(a, b); }
 __device__ __forceinline__ double dsub(double a, double b) { return __dsub_rn(a, b); }
-#endif
 // a / b with y = RN(1/b) precomputed: q = a*y; r = fma(-b,q,a); q' = fma(r,y,q).  Equals the IEEE
 // quotient except for the ~2^-51 fraction of dividends whose exact quotient sits within 1.7e-16 ulp of
 // a rounding boundary (see the header of this file); finite operands, no overflow / subnormal quotient.
 // A non-finite q (inf/NaN input or overflow) is returned as is, which is the IEEE result as well
 // (+-inf keeps its sign, NaN stays NaN) - branch free.
 __device__ __forceinline__ double ddiv_y(double a, double b, double y) {
-#ifdef GSB_FMA
-  (void)b;
-  return a * y;
-#endif
   const double q = __dmul_rn(a, y);
   const double r = __fma_rn(-b, q, a);
   const double q2 = __fma_rn(r, y, q);

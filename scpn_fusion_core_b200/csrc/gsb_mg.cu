@@ -136,7 +136,7 @@ int jacobi_steps_launch(gsb_ctx *ctx, double *psi, double *tmp, const double *sr
   const LevelGeom &g = ctx->levels[0].g;
   const size_t bytes = (size_t)batch * ctx->n * sizeof(double);
   double *cur = psi, *oth = tmp;
-  const bool fused_ok = g.nz >= 3 && g.nr >= 3 && !std::getenv("GSB_NO_FUSED_JACOBI");
+  const bool fused_ok = g.nz >= 3 && g.nr >= 3;
   int left = n_steps;
   while (left > 0) {
     int rc;

@@ -21,10 +21,7 @@
 
 namespace gsb {
 
-#ifndef GSB_RES_THREADS
-#define GSB_RES_THREADS 512
-#endif
-constexpr int kResThreads = GSB_RES_THREADS;  // threads of a resident CTA (one CTA per SM): 16 warps at 128 registers
+constexpr int kResThreads = 512;  // threads of a resident CTA (one CTA per SM): 16 warps at 128 registers
 constexpr int kResMaxLevels = 12;
 constexpr int kResSmemMax = 232448;  // 227 KB opt-in dynamic shared memory per CTA on sm_100
 
@@ -85,10 +82,6 @@ __device__ __forceinline__ int split_index(int nz, int hw, int iz, int ir) {
 // ddiv_y (and to IEEE a/b) whenever the quotient is finite; a non-finite quotient comes out as NaN
 // instead of +-inf, which every caller treats the same way (non-finite => diverged).
 __device__ __forceinline__ double ddiv_yf(double a, double b, double y) {
-#ifdef GSB_FMA
-  (void)b;
-  return a * y;
-#endif
   const double q = __dmul_rn(a, y);
   const double r = __fma_rn(-b, q, a);
   return __fma_rn(r, y, q);
@@ -184,7 +177,7 @@ __device__ __forceinline__ void res_smooth_run(int po, int qo, int ro, int hw, i
 // The same pass with the right-hand side of ALL rows of the run (at most kResMaxRun) already in
 // registers: the caller issues those global loads a whole pass ahead, so their L2 latency hides
 // behind the previous pass.  Fully unrolled over groups of four rows (compile-time register indices).
-constexpr int kResMaxRun = GSB_RES_THREADS >= 512 ? 16 : (GSB_RES_THREADS >= 384 ? 24 : 32);  // rows per thread on the finest level
+constexpr int kResMaxRun = 16;  // rows per thread on the finest level
 template <int S0>
 __device__ __forceinline__ void res_smooth_run_pref(int po, int qo, int hw, int cnt, double aeA, double awA, bool okA,
                                                     double aeB, double awB, bool okB, const SorK &c,

@@ -13,13 +13,10 @@
 // Strips/bands overlap by 2S columns/rows; the overlap is recomputed (an update is valid t+1 points
 // inside the tile edge after pass t) and only tile interiors are written, so with more than one
 // tile per equilibrium the sweep is out of place (neighbours read each other's interiors).
-// Two bodies implement this (bit-identical):
-//   sweep_warp_body_rc (default)  the lane's own values travel in registers, the shared-memory ring (rows as two half
-//                                 rows, even / odd columns, filled by cp.async) is landing zone + neighbour mailbox;
-//   sweep_warp_body               every operand is read from the ring (the r1 / early r2 form, kept as the measured
-//                                 comparison: GSB_SWEEP_UNROLL=2|4).
-// Arithmetic: the same operand order as sor_point (bit-identical results).  History and captures:
-// profiles/r2_sweep_icache.md.
+// The body, sweep_warp_body_rc, carries the lane's own values in registers; the shared-memory ring (rows as two half
+// rows, even / odd columns, filled by cp.async) is the landing zone of the row copies and the neighbour mailbox.
+// Arithmetic: the same operand order as sor_point (bit-identical results).  History and captures, including the form
+// that read every operand from the ring (bit-identical, 1.4-1.7x slower): profiles/r2_sweep_icache.md.
 #include "gsb_internal.cuh"
 
 namespace gsb {
@@ -46,9 +43,6 @@ __device__ __forceinline__ void cp_async_wait() {
   asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
 }
 
-// P0 = (zl + par_off + cl) & 1 of the warp's tile, hoisted into a template parameter by the
-// dispatching kernel below: with the step loop unrolled over one ring period every ring slot and
-// every colour parity is a compile-time constant (no address arithmetic in the loop body).
 // 32-bit shared-window accesses (the ring addresses rotate through registers, so the compiler could not prove the
 // address space of a generic pointer).  asm volatile keeps the program order of ring reads and writes.
 __device__ __forceinline__ double lds64(unsigned a) {
@@ -56,7 +50,6 @@ __device__ __forceinline__ double lds64(unsigned a) {
   asm volatile("ld.shared.f64 %0, [%1];" : "=d"(v) : "r"(a));
   return v;
 }
-__device__ __forceinline__ void sts64(unsigned a, double v) { asm volatile("st.shared.f64 [%0], %1;" ::"r"(a), "d"(v)); }
 __device__ __forceinline__ void sts64_if(bool p, unsigned a, double v) {  // predicated store, no branch
   asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.s32 p, %2, 0;\n\t@p st.shared.f64 [%0], %1;\n\t}" ::"r"(a), "d"(v), "r"((int)p));
 }
@@ -64,146 +57,11 @@ __device__ __forceinline__ void cp_async8s(unsigned s, const void *gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(s), "l"(gmem) : "memory");
 }
 
-// One warp, one tile.  P0 = (zl + par_off + cl) & 1 of the tile, hoisted into a template parameter by the dispatching
-// kernel below, UNR = steps per unrolled loop body (even, so every colour parity in the body is a compile-time constant).
-//
-// r1 unrolled the step loop over the whole ring period (16 steps): every ring slot was a compile-time constant, but the
-// body of the 6-stage kernel was 4 150 SASS instructions per parity variant (133 KB for both) with every warp of an SM
-// somewhere else in it, and ncu's top stall reason was `no_instruction` - instruction-cache misses (2.7 of 7.5 stalled
-// warp-cycles per issue, profiles/r2_sweep_icache.md).  Now the body is UNR = 2 steps and the sixteen slot addresses live
-// in sixteen registers that ROTATE by UNR after every body (A[i] = shared address of the slot that holds relative row
-// base - 11 + i): the wrap-around of the ring costs UNR register moves per step and no address arithmetic, row pointers
-// into global memory advance by one row per step instead of being recomputed.
-template <int NST, int P0, int UNR>
-__device__ __forceinline__ void sweep_warp_body(const SweepArgs &a, double *ring, int lane, int zl,
-                                                int zh, int z0, int z1, int cl, int wb, int c0, int c1,
-                                                const double *gin, const double *gsrc, double *gout) {
-  constexpr int NRING = 16;            // rows qi-2(NST-1)-1 .. qi+PF live at step qi
-  constexpr int PF = NRING - 2 * NST;  // prefetch distance in rows (deeper for the shorter steps of small NST)
-  constexpr unsigned SLOT = 64 * 8;    // bytes per ring slot: [even half row][odd half row] of 32 doubles
-  constexpr unsigned HALF = 32 * 8;
-  constexpr unsigned SRC = NRING * SLOT;  // the source ring follows the psi ring
-  static_assert(UNR % 2 == 0 && NRING % UNR == 0, "the unroll factor must keep the colour parity compile-time");
-  const int nr = a.nr;
-  const int xe = 2 * lane, xo = 2 * lane + 1;  // the lane's columns inside the strip
-  const bool have_e = xe < wb, have_o = xo < wb;
-  const bool upd_e = xe >= 1 && xe <= wb - 2, upd_o = xo <= wb - 2;
-  const bool wr_e = have_e && cl + xe >= c0 && cl + xe < c1, wr_o = have_o && cl + xo >= c0 && cl + xo < c1;
-  const double ae_e = have_e ? a.a_e[cl + xe] : 0.0, aw_e = have_e ? a.a_w[cl + xe] : 0.0;
-  const double ae_o = have_o ? a.a_e[cl + xo] : 0.0, aw_o = have_o ? a.a_w[cl + xo] : 0.0;
-  const double a_ns = a.a_ns, a_c = a.a_c, inv_a_c = a.inv_a_c, omega = a.omega, omw = a.omw;
-  const unsigned rb = (unsigned)__cvta_generic_to_shared(ring) + (unsigned)lane * 8u;  // slot 0, even half, this lane
-  const int nrows = zh - zl;   // loaded rows, relative index q = r - zl in [0, nrows)
-  const size_t rowb = (size_t)nr * sizeof(double);
-
-  // asynchronous copy of one row (psi and source) into the slot at shared address `sa`; `pr` / `sr` point at this
-  // lane's even column of that row
-  auto load_row = [&](bool row_ok, unsigned sa, const char *pr, const char *sr) {
-    if (row_ok) {
-      if (have_e) {
-        cp_async8s(sa, pr);
-        cp_async8s(sa + SRC, sr);
-      }
-      if (have_o) {
-        cp_async8s(sa + HALF, pr + 8);
-        cp_async8s(sa + SRC + HALF, sr + 8);
-      }
-    }
-    cp_async_commit();
-  };
-  const char *pin = (const char *)(gin + (size_t)zl * nr + cl + xe);
-  const char *psr = (const char *)(gsrc + (size_t)zl * nr + cl + xe);
-#pragma unroll
-  for (int q = 0; q <= PF; ++q) load_row(q < nrows, rb + q * SLOT, pin + q * rowb, psr + q * rowb);
-  pin += (size_t)(PF + 1) * rowb;  // the row step qi = 1 prefetches
-  psr += (size_t)(PF + 1) * rowb;
-  cp_async_wait<PF - 2>();  // rows 0 .. 2 have landed
-  __syncwarp();
-
-  unsigned A[NRING];  // A[i]: slot of relative row base - 11 + i, i.e. slot (base + i + 5) & 15
-#pragma unroll
-  for (int i = 0; i < NRING; ++i) A[i] = rb + ((i + 5) & (NRING - 1)) * SLOT;
-  // row written back at step qi is relative row qi - 2(NST-1); pointer at this lane's even column, for qi = 1
-  char *pout = (char *)(gout + cl + xe) + ((ptrdiff_t)zl + 1 - 2 * (NST - 1)) * (ptrdiff_t)rowb;
-  const unsigned w_lo = (unsigned)(z0 - zl + 2 * (NST - 1)), w_n = (unsigned)(z1 - z0);  // write iff qi - w_lo < w_n (unsigned)
-  const unsigned q_hi = (unsigned)(nrows - 3);  // a stage row q is updated iff (unsigned)(q - 1) <= q_hi
-  const int q_end = (nrows - 2) + 2 * (NST - 1);  // last step (relative row of stage 0)
-  for (int base = 0; base <= q_end; base += UNR) {
-#pragma unroll
-    for (int u = 0; u < UNR; ++u) {
-      const int qi = base + u;  // stage 0 is at relative row qi (row 0 is never updated)
-      if (qi >= 1 && qi <= q_end) {
-        double W[NST], E[NST], S[NST], N[NST], O[NST], F[NST], V[NST];
-        // ---- operands of every stage (stage t = colour pass t at relative row qi - 2t = ring index 11 + u - 2t)
-#pragma unroll
-        for (int t = 0; t < NST; ++t) {
-          const int hx = (t + u + P0) & 1;  // column parity of this pass's points in that row (compile time)
-          const unsigned me = A[(11 + u - 2 * t) & (NRING - 1)] + hx * HALF;        // own half row
-          const unsigned ot = A[(11 + u - 2 * t) & (NRING - 1)] + (1 - hx) * HALF;  // the other colour's half row
-          // unconditional loads (always inside the ring): no branches, so the 2S stages overlap
-          W[t] = lds64(hx ? ot : ot - 8);
-          E[t] = lds64(hx ? ot + 8 : ot);
-          S[t] = lds64(A[(10 + u - 2 * t) & (NRING - 1)] + hx * HALF);
-          N[t] = lds64(A[(12 + u - 2 * t) & (NRING - 1)] + hx * HALF);
-          O[t] = lds64(me);
-          F[t] = lds64(me + SRC);
-        }
-        // ---- 2S independent updates
-#pragma unroll
-        for (int t = 0; t < NST; ++t) {
-          const int hx = (t + u + P0) & 1;
-          double acc = dadd(dmul(hx ? ae_o : ae_e, E[t]), dmul(hx ? aw_o : aw_e, W[t]));
-          acc = dadd(acc, dmul(a_ns, S[t]));
-          acc = dadd(acc, dmul(a_ns, N[t]));
-          acc = dsub(acc, F[t]);
-          const double qq = __dmul_rn(acc, inv_a_c);
-          const double gs = __fma_rn(__fma_rn(-a_c, qq, acc), inv_a_c, qq);  // acc / a_c (Markstein sequence, gsb_internal.cuh)
-          V[t] = dadd(dmul(omw, O[t]), dmul(omega, gs));
-        }
-#pragma unroll
-        for (int t = 0; t < NST; ++t) {
-          const int hx = (t + u + P0) & 1;
-          const bool on = ((unsigned)(qi - 2 * t - 1) <= q_hi) && (hx ? upd_o : upd_e);
-          if (on) sts64(A[(11 + u - 2 * t) & (NRING - 1)] + hx * HALF, V[t]);
-        }
-        load_row(qi + PF < nrows, A[(11 + u + PF) & (NRING - 1)], pin, psr);
-        pin += rowb;
-        psr += rowb;
-        cp_async_wait<PF - 2>();  // row qi+2 has landed (stage 0 of the next step reads it)
-        __syncwarp();
-        // ---- relative row qi - 2(NST-1) is final once the last pass has processed it: write the tile interior back
-        if ((unsigned)qi - w_lo < w_n) {
-          const unsigned sa = A[(11 + u - 2 * (NST - 1)) & (NRING - 1)];
-          if (wr_e) *(double *)pout = lds64(sa);
-          if (wr_o) *(double *)(pout + 8) = lds64(sa + HALF);
-        }
-        pout += rowb;
-      }
-    }
-    // the ring moves on by UNR rows
-    unsigned head[UNR];
-#pragma unroll
-    for (int i = 0; i < UNR; ++i) head[i] = A[i];
-#pragma unroll
-    for (int i = 0; i + UNR < NRING; ++i) A[i] = A[i + UNR];
-#pragma unroll
-    for (int i = 0; i < UNR; ++i) A[NRING - UNR + i] = head[i];
-  }
-  // rows that no stage ever processes (next to the array edge: walls / halo rows)
-  if (gout != gin) {
-    for (int w = z0; w < z1; ++w) {
-      if (w >= zl + 1 && w <= zh - 2) continue;
-      const double *irow = gin + (size_t)w * nr + cl;
-      double *orow = gout + (size_t)w * nr + cl;
-      if (wr_e) orow[xe] = irow[xe];
-      if (wr_o) orow[xo] = irow[xo];
-    }
-  }
-}
-
-// Register-carried variant (the "register blocking" of the smoother).  A lane owns the column pair (2k, 2k+1) of the
-// strip, and of the five neighbours of an update only ONE belongs to another lane (west of the even column / east of the
-// odd one); everything else the same lane produced itself a few steps earlier:
+// One warp, one tile, register-carried (the "register blocking" of the smoother).  P0 = (zl + par_off + cl) & 1 of the
+// tile, hoisted into a template parameter by the dispatching kernel below, keeps every colour parity in the unrolled
+// loop body a compile-time constant.  A lane owns the column pair (2k, 2k+1) of the strip, and of the five neighbours
+// of an update only ONE belongs to another lane (west of the even column / east of the odd one); everything else the
+// same lane produced itself a few steps earlier:
 //   stage t at step qi updates (row q = qi - 2t, half hx):   K_t(qi) := the point's value afterwards (V, or O if masked)
 //     N     = (q+1, hx)    = K_{t-1}(qi-1)        S = (q-1, hx) = K_{t-1}(qi-3)
 //     own W/E = (q, 1-hx)  = K_{t-1}(qi-2)        O = (q, hx)   = K_{t-2}(qi-4)      F = source(q, hx) = F_{t-2}(qi-4)
@@ -211,9 +69,10 @@ __device__ __forceinline__ void sweep_warp_body(const SweepArgs &a, double *ring
 //     its own W/E = a(qi-1), S = a(qi-2);  stage 1's O = a(qi-3).
 // With the step loop unrolled by 4 every carried value has a fixed register name (index = step & 3), so the ring in
 // shared memory is only the landing zone of the asynchronous row copies and the mailbox for the one neighbour value:
-// 10 shared loads + 5 stores per step instead of 42 + 6 (the r2 kernel ran the shared-memory pipe at 74 %,
-// profiles/r2_sweep_icache.md), and finished rows go from registers straight to global memory.
-// The arithmetic and its order are those of the ring kernel: results are bit-identical.
+// 10 shared loads + 5 stores per step instead of the 42 + 6 of reading every operand from the ring (which ran the
+// shared-memory pipe at 74 %, profiles/r2_sweep_icache.md), and finished rows go from registers straight to global
+// memory.  The loop is unrolled by 4 steps, not over the whole 16-row ring period (that body missed the instruction
+// cache), so the sixteen slot addresses live in sixteen registers that rotate by UNR after every loop body.
 template <int NST, int P0>
 __device__ __forceinline__ void sweep_warp_body_rc(const SweepArgs &a, double *ring, int lane, int zl,
                                                    int zh, int z0, int z1, int cl, int wb, int c0, int c1,
@@ -364,7 +223,7 @@ __device__ __forceinline__ void sweep_warp_body_rc(const SweepArgs &a, double *r
   }
 }
 
-template <int NST, int UNR>
+template <int NST>
 __global__ void __launch_bounds__(32 * kSwWPC) k_sweep_warp(const SweepArgs a) {
   constexpr int NRING = 16;
   constexpr int STEP = kSwCols - 2 * NST;  // interior columns per strip (even)
@@ -390,17 +249,10 @@ __global__ void __launch_bounds__(32 * kSwWPC) k_sweep_warp(const SweepArgs a) {
   const double *gin = a.in + (size_t)b * a.istride;
   const double *gsrc = a.src + (size_t)b * a.sstride;
   double *gout = a.out + (size_t)b * a.ostride;
-  if constexpr (UNR == 1) {  // register-carried variant
-    if ((zl + a.par_off + cl) & 1)
-      sweep_warp_body_rc<NST, 1>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
-    else
-      sweep_warp_body_rc<NST, 0>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
-  } else {
-    if ((zl + a.par_off + cl) & 1)
-      sweep_warp_body<NST, 1, UNR>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
-    else
-      sweep_warp_body<NST, 0, UNR>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
-  }
+  if ((zl + a.par_off + cl) & 1)
+    sweep_warp_body_rc<NST, 1>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
+  else
+    sweep_warp_body_rc<NST, 0>(a, ring, lane, zl, zh, z0, z1, cl, wb, c0, c1, gin, gsrc, gout);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -609,9 +461,8 @@ __global__ void __launch_bounds__(32 * kSwWPC, 3) k_jacobi_warp(const SweepArgs 
                       a.src + (size_t)b * a.sstride, a.out + (size_t)b * a.ostride);
 }
 
-static size_t sweep_smem_bytes(int nst) {
+static size_t sweep_smem_bytes() {
   const int nring = 16;
-  (void)nst;
   return (size_t)(kSwWPC * 2 * nring * kSwCols) * sizeof(double);
 }
 
@@ -672,32 +523,19 @@ int sweep_fused_launch(const LevelGeom &g, const double *in, size_t istride, dou
   a.omega = omega;
   a.omw = 1.0 - omega;
   a.active = active;
-  const size_t smem = sweep_smem_bytes(nst);
+  const size_t smem = sweep_smem_bytes();
   const dim3 grd((ns * nb + kSwWPC - 1) / kSwWPC, 1, batch), blk(32 * kSwWPC, 1, 1);
-  static const int unroll = [] {  // 1 (default) = register-carried kernel; measurement switch: 2 / 4 = ring kernel with that many steps per loop body
-    const char *e = std::getenv("GSB_SWEEP_UNROLL");
-    const int v = e ? std::atoi(e) : 1;
-    return (v == 1 || v == 2 || v == 4) ? v : 1;
-  }();
-#define GSB_SWEEP_LAUNCH(NST_, UNR_)                                   \
-  do {                                                                 \
-    GSB_SMEM_OPT_IN((k_sweep_warp<NST_, UNR_>), smem);                 \
-    k_sweep_warp<NST_, UNR_><<<grd, blk, smem, st>>>(a);               \
-  } while (0)
-#define GSB_SWEEP_DISPATCH(NST_)                                       \
-  do {                                                                 \
-    if (unroll == 4) GSB_SWEEP_LAUNCH(NST_, 4);                        \
-    else if (unroll == 1) GSB_SWEEP_LAUNCH(NST_, 1);                   \
-    else GSB_SWEEP_LAUNCH(NST_, 2);                                    \
-  } while (0)
-  if (nst == 2)
-    GSB_SWEEP_DISPATCH(2);
-  else if (nst == 4)
-    GSB_SWEEP_DISPATCH(4);
-  else
-    GSB_SWEEP_DISPATCH(6);
-#undef GSB_SWEEP_DISPATCH
-#undef GSB_SWEEP_LAUNCH
+  // one GSB_SMEM_OPT_IN per kernel: each expansion remembers on its own that its attribute is set
+  if (nst == 2) {
+    GSB_SMEM_OPT_IN(k_sweep_warp<2>, smem);
+    k_sweep_warp<2><<<grd, blk, smem, st>>>(a);
+  } else if (nst == 4) {
+    GSB_SMEM_OPT_IN(k_sweep_warp<4>, smem);
+    k_sweep_warp<4><<<grd, blk, smem, st>>>(a);
+  } else {
+    GSB_SMEM_OPT_IN(k_sweep_warp<6>, smem);
+    k_sweep_warp<6><<<grd, blk, smem, st>>>(a);
+  }
   GSB_LAUNCH_CHECK();
   return GSB_OK;
 }
@@ -711,14 +549,8 @@ int jacobi_fused_launch(const LevelGeom &g, const double *in, double *out, const
   SweepArgs a{};
   a.nz = g.nz;
   a.nr = g.nr;
-  // strips of 64 - 2T interior columns; bands as for the sweeps (T halo rows per side)
-  const int step = kSwCols - 2 * T;
-  const int ns = g.nr <= kSwCols ? 1 : (g.nr + step - 1) / step;
-  const long long warps = (long long)ns * batch, want = 24LL * num_sms;
-  int bands = 1;
-  if (warps < want) bands = (int)std::min<long long>((want + warps - 1) / warps, std::max(1, g.nz / 8));
-  a.band_rows = (g.nz + bands - 1) / bands;
-  const int nb = (g.nz + a.band_rows - 1) / a.band_rows;
+  int ns, nb, sc;  // T halo rows / columns per side, like a sweep of T stages
+  sweep_fused_plan(g.nz, g.nr, batch, T, num_sms, &sc, &a.band_rows, &ns, &nb);
   a.n_strips = ns;
   a.n_bands = nb;
   a.in = in;
@@ -731,7 +563,7 @@ int jacobi_fused_launch(const LevelGeom &g, const double *in, double *out, const
   a.a_c = g.a_c;
   a.inv_a_c = g.inv_a_c;
   a.active = active;
-  const size_t smem = sweep_smem_bytes(0);
+  const size_t smem = sweep_smem_bytes();
   const dim3 grd((ns * nb + kSwWPC - 1) / kSwWPC, 1, batch), blk(32 * kSwWPC, 1, 1);
   GSB_SMEM_OPT_IN(k_jacobi_warp<T>, smem);
   k_jacobi_warp<T><<<grd, blk, smem, st>>>(a);

@@ -136,7 +136,7 @@ def test_plasma_wall_option_vs_numpy_restatement(pkg, n, wall_mu0):
     cfg = golden_cfg(golden("solves"), "iter65")
     cfg["grid_resolution"] = [n, n]
     cfg["physics"]["profiles"] = {"mode": "h-mode"}
-    B = 130 if n == 33 else 3  # >= 128 rows take k_wall_gemm_big, fewer the 64x64 kernel
+    B = 130 if n == 33 else 3  # k_wall_gemm_sk tiles the batch by 128: two tiles (the second ragged) or one ragged tile
     cc, ip, ped = _uq(cfg, B)
     bk = pkg.BatchedFusionKernel(cfg)
     r = bk.solve_free_boundary(cc, ip, ped, ped, max_outer_iter=4, tol=1e-6, plasma_wall=True, wall_mu0=wall_mu0)

@@ -38,14 +38,6 @@ for n, B in shapes:
     dA = float((R[1] - R[0]) * (Z[1] - Z[0]))
     run = lambda: _lib.check(ctx.lib.gsb_wall_flux(ctx.handle, D.ptr(M), D.ptr(J), dA, D.ptr(wall), B, st))
     flops = 2.0 * B * nw * ni
-    if os.environ.get("GSB_GEMM_SWEEP") and (n, B) == (129, 4096):
-        for v in (0, 1, 2, 3):
-            os.environ["GSB_GEMM_VARIANT"] = str(v)
-            msv = timeit(run)
-            Xv = (J[:, 1:-1, 1:-1].reshape(B, ni) * dA)
-            errv = float((wall - Xv @ M.T).abs().max())
-            print(json.dumps({"variant": v, "ms": msv, "tflops": flops / msv / 1e9, "abs_err": errv}), flush=True)
-        os.environ.pop("GSB_GEMM_VARIANT")
     ms = timeit(run)
     X = (J[:, 1:-1, 1:-1].reshape(B, ni) * dA).contiguous()
     ref = X @ M.T
