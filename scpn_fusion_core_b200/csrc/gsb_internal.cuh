@@ -388,4 +388,16 @@ int ring_save_launch(const double *f, size_t stride, double *ring, int nz, int n
 int residual_norms_launch(gsb_ctx *ctx, const LevelGeom &g, const double *psi, size_t pstride,
                           const double *src, size_t sstride, double *linf, double *rms, int batch,
                           const int *active, cudaStream_t st);
+// The seam between the batched free-boundary loop (gsb_picard.cu) and its shape step (gsb_fit.cu), kept out of the
+// library's exports.  free_boundary_loop runs the shape step `sh` after every inner solve unless sh is NULL.
+#pragma GCC visibility push(hidden)
+struct ShapeStep;
+int free_boundary_check(gsb_ctx *ctx, const gsb_free_boundary_params *fb, int batch);
+int free_boundary_loop(gsb_ctx *ctx, const gsb_picard_params *p, const gsb_free_boundary_params *fb, const ShapeStep *sh,
+                       double *psi_dev, double *psi_ext_dev, const double *wall_m_dev, const double *ip_dev,
+                       const double *prof_dev, double *jphi_dev, double *summary_dev, double *fb_summary_dev, int batch,
+                       void *stream);
+int shape_step_launch(gsb_ctx *ctx, const ShapeStep &sh, const double *psi, double *psi_ext, const int *mask, int batch,
+                      cudaStream_t st);
+#pragma GCC visibility pop
 }  // namespace gsb
