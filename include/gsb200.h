@@ -289,6 +289,43 @@ int gsb_probe_reconstruct(const gsb_probe_params *pp, const double *meas_dev, co
                           double *currents_dev, double *residual_dev, double *wresidual_dev, double *stats_dev,
                           void *work_dev, long long *work_bytes, int batch, void *stream);
 
+typedef struct gsb_boundary_params {
+  int n_coils;             /* 1..65535 */
+  const double *coil_rz;   /* HOST [n_coils][2] coil (R, Z) */
+  const int *turns;        /* HOST [n_coils] integer turns (>= 1) */
+  int n_points;            /* boundary points N, 1..4096 */
+  const double *points;    /* HOST [N][2] (R, Z) */
+  int n_limiter;           /* limiter points L, 0..4096 */
+  const double *limiter;   /* HOST [L][2] or NULL when L = 0 */
+  int has_axis;            /* 0 or 1 */
+  const double *axis;      /* HOST [2] ([batch][2] when per_sample) or NULL */
+  int n_xpoints;           /* X-points X, 0..64 */
+  const double *xpoints;   /* HOST [X][2] ([batch][X][2] when per_sample) or NULL when X = 0 */
+  int per_sample;          /* 1: the axis and X-points are given per sample */
+  int target_mode;         /* 0: no target; 1: target_dev [N]; 2: target_dev [batch][N]; 3: target_dev is a field
+                              [batch][nz][nr] read on its wall contour (fusion_kernel_free_boundary.py:608-620 order) */
+  int nz, nr;              /* target_mode 3: field shape */
+  const double *r_axis;    /* target_mode 3: HOST [nr] and [nz] grid axes; the N = 2 nr + 2 nz - 4 boundary points */
+  const double *z_axis;    /*                must be the wall contour of these axes, in its order */
+} gsb_boundary_params;
+
+/* reconstruct_boundary_flux_from_coils (fusion_kernel_free_boundary.py:162-267) for `batch` coil-current vectors.
+ * Context-free: it runs on the current device and `stream`.  The flux at a point p of sample b is
+ * sum_c M[c][p] I[b][c], accumulated in coil order from 0.0 without contraction, M[c][p] = turns_c G_SI(coil c -> p)
+ * (gsb_mutual_matrix), so it does not depend on the sample's batch position.
+ * currents_dev [batch][n_coils] coil currents in amperes
+ * target_dev   see target_mode (NULL when target_mode = 0)
+ * flux_dev     [batch][N + L + has_axis + X] out: boundary, limiter, axis and X-point flux, in that order
+ * residual_dev [batch][N] out: flux - target (NULL when target_mode = 0)
+ * stats_dev    [batch][5] out: rmse = sqrt(np.mean(residual**2)) (NumPy's pairwise order), max |residual|,
+ *              x_point_flux_span = max - min of the X-point flux, |xf0 - xf1| (X = 2), flags (1: a boundary flux is
+ *              not finite, 2: a target value is not finite); NaN where the value does not apply
+ * work_dev     device workspace of *work_bytes bytes; with work_dev NULL the call only stores the size it needs in
+ *              *work_bytes (the counts, per_sample and batch must then be set). */
+int gsb_boundary_flux(const gsb_boundary_params *bp, const double *currents_dev, const double *target_dev,
+                      double *flux_dev, double *residual_dev, double *stats_dev, void *work_dev, long long *work_bytes,
+                      int batch, void *stream);
+
 /* Measurement hook (bench.py roofline): while enabled, gsb_free_boundary_solve brackets every inner Picard solve and
  * every wall GEMM with CUDA events on the launching stream and accumulates
  * out4 = {Picard solves: total ms, count; wall GEMMs: total ms, count}.  out4 may be NULL; reset != 0 zeroes the sums. */

@@ -46,6 +46,14 @@ class gsb_probe_params(ctypes.Structure):
                 ("alpha", c_double), ("limits", POINTER(c_double)), ("max_iter", c_int)]
 
 
+class gsb_boundary_params(ctypes.Structure):
+    _fields_ = [("n_coils", c_int), ("coil_rz", POINTER(c_double)), ("turns", POINTER(c_int)), ("n_points", c_int),
+                ("points", POINTER(c_double)), ("n_limiter", c_int), ("limiter", POINTER(c_double)),
+                ("has_axis", c_int), ("axis", POINTER(c_double)), ("n_xpoints", c_int), ("xpoints", POINTER(c_double)),
+                ("per_sample", c_int), ("target_mode", c_int), ("nz", c_int), ("nr", c_int),
+                ("r_axis", POINTER(c_double)), ("z_axis", POINTER(c_double))]
+
+
 _dp = POINTER(c_double)
 _ip = POINTER(c_int)
 
@@ -96,6 +104,8 @@ SIGNATURES = {
                                               c_void_p, c_int, c_void_p]),
     "gsb_probe_reconstruct": (c_int, [POINTER(gsb_probe_params), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                                       c_void_p, c_void_p, POINTER(c_longlong), c_int, c_void_p]),
+    "gsb_boundary_flux": (c_int, [POINTER(gsb_boundary_params), c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
+                                  c_void_p, POINTER(c_longlong), c_int, c_void_p]),
     "gsb_enable_peer_access": (c_int, [c_int, c_int]),
     "gsb_ipc_alloc": (c_int, [c_int, c_longlong, POINTER(c_void_p), c_char_p]),
     "gsb_ipc_open": (c_int, [c_int, c_char_p, POINTER(c_void_p)]),

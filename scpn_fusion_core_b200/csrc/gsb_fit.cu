@@ -456,6 +456,103 @@ __global__ void __launch_bounds__(32 * kShapeWarps) k_probe_fit(ProbeFitArgs g) 
   }
 }
 
+// ---------------------------------------------------------------------------- wall-contour boundary reconstruction
+// (reconstruct_boundary_flux_from_coils, fusion_kernel_free_boundary.py:162-267).  One CTA per sample: the coil flux at
+// every boundary, limiter, axis and X-point point, then the residual against the target and its reductions in fixed
+// orders (no atomics), so a sample's bits do not depend on its batch position.
+constexpr int kBoundaryMaxPoints = 4096;
+constexpr int kBoundaryMaxX = 64;
+constexpr int kBoundaryThreads = 256;
+
+struct BoundaryArgs {
+  const double *m;       // [nc][ncol] turns * G_SI: shared columns, then [batch][A + X] per-sample columns
+  const double *cur;     // [B][nc]
+  const double *target;  // NULL, [N], [B][N] or [B][nz][nr]
+  double *flux;          // [B][N + L + A + X]
+  double *residual;      // [B][N]
+  double *stats;         // [B][5]
+  int nc, ncol, n_shared, N, L, A, X, per_sample, target_mode, nz, nr;
+};
+
+// offset in a [nz][nr] field of wall-contour point p (_wall_contour: bottom row left to right, right column upwards,
+// top row right to left, left column downwards)
+__device__ __forceinline__ int wall_contour_offset(int p, int nz, int nr) {
+  if (p < nr) return p;
+  p -= nr;
+  if (p < nz - 1) return (p + 1) * nr + nr - 1;
+  p -= nz - 1;
+  if (p < nr - 1) return (nz - 1) * nr + nr - 2 - p;
+  p -= nr - 1;
+  return (nz - 2 - p) * nr;
+}
+
+// np.max's rule: the larger value, and a NaN sticks
+__device__ __forceinline__ double nan_max(double a, double b) { return (b > a || b != b) && a == a ? b : a; }
+
+__global__ void __launch_bounds__(kBoundaryThreads) k_boundary_flux(BoundaryArgs g) {
+  __shared__ double sq[kBoundaryMaxPoints];
+  __shared__ double xf[kBoundaryMaxX];
+  __shared__ double wmax[kBoundaryThreads / 32];
+  const int b = blockIdx.x, tid = threadIdx.x;
+  const int NL = g.N + g.L, nout = NL + g.A + g.X;
+  const double *cb = g.cur + (size_t)b * g.nc;
+  double *fb = g.flux + (size_t)b * nout;
+  double mx = 0.0;
+  int rec_bad = 0, tgt_bad = 0;
+  for (int p = tid; p < nout; p += blockDim.x) {
+    const int col = (p >= NL && g.per_sample) ? g.n_shared + b * (g.A + g.X) + (p - NL) : p;
+    double acc = 0.0;
+    for (int c = 0; c < g.nc; ++c) acc = dadd(acc, dmul(g.m[(size_t)c * g.ncol + col], cb[c]));
+    fb[p] = acc;
+    if (p >= NL + g.A) xf[p - NL - g.A] = acc;
+    if (p < g.N) {
+      rec_bad |= !isfinite(acc);
+      if (g.target_mode) {
+        const double t = g.target_mode == 1   ? g.target[p]
+                         : g.target_mode == 2 ? g.target[(size_t)b * g.N + p]
+                                              : g.target[(size_t)b * g.nz * g.nr + wall_contour_offset(p, g.nz, g.nr)];
+        tgt_bad |= !isfinite(t);
+        const double r = dsub(acc, t);
+        g.residual[(size_t)b * g.N + p] = r;
+        sq[p] = dmul(r, r);
+        mx = nan_max(mx, fabs(r));
+      }
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) mx = nan_max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if ((tid & 31) == 0) wmax[tid >> 5] = mx;
+  rec_bad = __syncthreads_or(rec_bad);
+  tgt_bad = __syncthreads_or(tgt_bad);
+  if (tid != 0) return;
+  double *s = g.stats + (size_t)b * 5;
+  if (g.target_mode) {
+    for (int w = 1; w < (int)(blockDim.x >> 5); ++w) mx = nan_max(mx, wmax[w]);
+    s[0] = __dsqrt_rn(__ddiv_rn(np_pairwise_dev<6>(sq, g.N), (double)g.N));  // depth 6 covers kBoundaryMaxPoints
+    s[1] = mx;
+  } else {
+    s[0] = s[1] = NAN;
+  }
+  double hi = NAN, lo = NAN;
+  if (g.X) {
+    hi = lo = xf[0];
+    for (int k = 1; k < g.X; ++k) {
+      hi = nan_max(hi, xf[k]);
+      lo = -nan_max(-lo, -xf[k]);
+    }
+  }
+  s[2] = g.X ? dsub(hi, lo) : NAN;
+  s[3] = g.X == 2 ? fabs(dsub(xf[0], xf[1])) : NAN;
+  s[4] = (double)(rec_bad + 2 * tgt_bad);
+}
+
+// finite (R, Z) with R > 0 for every one of n points
+static bool points_ok(const double *rz, long long n) {
+  for (long long i = 0; i < n; ++i)
+    if (!std::isfinite(rz[2 * i]) || !std::isfinite(rz[2 * i + 1]) || !(rz[2 * i] > 0.0)) return false;
+  return true;
+}
+
 // The shape step of gsb_free_boundary_shape_solve (device workspace laid out by that entry)
 struct ShapeStep {
   ShapeFitArgs fit;
@@ -688,6 +785,98 @@ int gsb_probe_reconstruct(const gsb_probe_params *pp, const double *meas_dev, co
   a.batch = batch;
   a.max_iter = pp->max_iter > 0 ? pp->max_iter : 3 * n + 10;
   k_probe_fit<<<(batch + kShapeWarps - 1) / kShapeWarps, 32 * kShapeWarps, 0, st>>>(a);
+  GSB_LAUNCH_CHECK();
+  return GSB_OK;
+}
+
+int gsb_boundary_flux(const gsb_boundary_params *bp, const double *currents_dev, const double *target_dev,
+                      double *flux_dev, double *residual_dev, double *stats_dev, void *work_dev, long long *work_bytes,
+                      int batch, void *stream) {
+  // every argument is checked here, before the first launch
+  GSB_REQUIRE(bp && work_bytes, "gsb_boundary_flux: NULL argument");
+  const int nc = bp->n_coils, N = bp->n_points, L = bp->n_limiter, A = bp->has_axis, X = bp->n_xpoints;
+  GSB_REQUIRE(nc >= 1 && nc <= 65535, "boundary reconstruction supports 1 to 65535 coils on the device.");
+  GSB_REQUIRE(N >= 1 && N <= kBoundaryMaxPoints, "boundary reconstruction supports 1 to 4096 boundary points.");
+  GSB_REQUIRE(L >= 0 && L <= kBoundaryMaxPoints, "boundary reconstruction supports at most 4096 limiter points.");
+  GSB_REQUIRE(A == 0 || A == 1, "gsb_boundary_flux: has_axis must be 0 or 1");
+  GSB_REQUIRE(X >= 0 && X <= kBoundaryMaxX, "boundary reconstruction supports at most 64 X-points.");
+  GSB_REQUIRE(bp->per_sample == 0 || bp->per_sample == 1, "gsb_boundary_flux: per_sample must be 0 or 1");
+  GSB_REQUIRE(bp->target_mode >= 0 && bp->target_mode <= 3, "gsb_boundary_flux: target_mode must be 0..3");
+  GSB_REQUIRE(batch >= 1, "gsb_boundary_flux: batch must be >= 1");
+  // point columns of M: boundary | limiter | axis, X-points (once, or once per sample)
+  const long long n_shared = (long long)N + L + (bp->per_sample ? 0 : A + X);
+  const long long n_own = bp->per_sample ? (long long)batch * (A + X) : 0;
+  GSB_REQUIRE(n_shared + n_own <= 0x7fffffffLL, "gsb_boundary_flux: too many point evaluations for one call");
+  const long long ncol = n_shared + n_own;
+  const size_t need = (size_t)nc * (size_t)ncol * sizeof(double);
+  if (!work_dev) {
+    *work_bytes = (long long)need;
+    return GSB_OK;
+  }
+  GSB_REQUIRE(*work_bytes >= (long long)need, "gsb_boundary_flux: workspace too small");
+  GSB_REQUIRE(currents_dev && flux_dev && stats_dev && bp->coil_rz && bp->turns && bp->points,
+              "gsb_boundary_flux: NULL argument");
+  GSB_REQUIRE(!bp->target_mode || (target_dev && residual_dev), "gsb_boundary_flux: a target needs target_dev and "
+                                                                "residual_dev");
+  GSB_REQUIRE((!L || bp->limiter) && (!A || bp->axis) && (!X || bp->xpoints), "gsb_boundary_flux: NULL point array");
+  GSB_REQUIRE(points_ok(bp->coil_rz, nc), "source coil coordinates must be finite with R_src > 0.");
+  for (int c = 0; c < nc; ++c) GSB_REQUIRE(bp->turns[c] >= 1, "turns must be positive integers.");
+  const long long n_ax = bp->per_sample ? (long long)batch * A : A, n_x = bp->per_sample ? (long long)batch * X : X;
+  GSB_REQUIRE(points_ok(bp->points, N) && (!L || points_ok(bp->limiter, L)) && (!A || points_ok(bp->axis, n_ax)) &&
+                  (!X || points_ok(bp->xpoints, n_x)),
+              "boundary, limiter, axis and X-point coordinates must be finite with positive radii.");
+  const int nz = bp->nz, nr = bp->nr;
+  if (bp->target_mode == 3) {
+    GSB_REQUIRE(nz >= 2 && nr >= 2 && bp->r_axis && bp->z_axis, "gsb_boundary_flux: the wall-contour target needs "
+                                                                "nz, nr >= 2 and both grid axes");
+    GSB_REQUIRE(N == 2 * nr + 2 * nz - 4, "the wall-contour target needs N = 2 nr + 2 nz - 4 boundary points.");
+    bool same = true;
+    for (int p = 0; p < N && same; ++p) {
+      int iz, ir;  // _wall_contour's (iz, ir) of point p (the order of wall_contour_offset)
+      if (p < nr) iz = 0, ir = p;
+      else if (p < nr + nz - 1) iz = p - nr + 1, ir = nr - 1;
+      else if (p < 2 * nr + nz - 2) iz = nz - 1, ir = 2 * nr + nz - 3 - p;
+      else iz = 2 * nr + 2 * nz - 4 - p, ir = 0;
+      same = bp->points[2 * p] == bp->r_axis[ir] && bp->points[2 * p + 1] == bp->z_axis[iz];
+    }
+    GSB_REQUIRE(same, "the wall-contour target needs the wall contour of the grid as boundary points.");
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  std::vector<double> obs(2 * (size_t)ncol);
+  double *o = obs.data();
+  o = std::copy(bp->points, bp->points + 2 * (size_t)N, o);
+  if (L) o = std::copy(bp->limiter, bp->limiter + 2 * (size_t)L, o);
+  if (bp->per_sample) {
+    for (int b = 0; b < batch; ++b) {
+      if (A) o = std::copy(bp->axis + 2 * (size_t)b, bp->axis + 2 * (size_t)b + 2, o);
+      if (X) o = std::copy(bp->xpoints + 2 * (size_t)b * X, bp->xpoints + 2 * ((size_t)b + 1) * X, o);
+    }
+  } else {
+    if (A) o = std::copy(bp->axis, bp->axis + 2, o);
+    if (X) o = std::copy(bp->xpoints, bp->xpoints + 2 * (size_t)X, o);
+  }
+  double *d_m = (double *)work_dev;
+  int rc = gsb_mutual_matrix(bp->coil_rz, bp->turns, nc, obs.data(), (int)ncol, d_m, stream);
+  if (rc) return rc;
+  BoundaryArgs a{};
+  a.m = d_m;
+  a.cur = currents_dev;
+  a.target = target_dev;
+  a.flux = flux_dev;
+  a.residual = residual_dev;
+  a.stats = stats_dev;
+  a.nc = nc;
+  a.ncol = (int)ncol;
+  a.n_shared = (int)n_shared;
+  a.N = N;
+  a.L = L;
+  a.A = A;
+  a.X = X;
+  a.per_sample = bp->per_sample;
+  a.target_mode = bp->target_mode;
+  a.nz = nz;
+  a.nr = nr;
+  k_boundary_flux<<<batch, kBoundaryThreads, 0, st>>>(a);
   GSB_LAUNCH_CHECK();
   return GSB_OK;
 }

@@ -336,6 +336,21 @@ def _wall_contour(kernel: Any):
     return np.column_stack([r[ir], z[iz]]), iz, ir
 
 
+def _limiter_geometry(obs: np.ndarray, lim: np.ndarray) -> dict[str, Any]:
+    """The geometry-only limiter keys of reconstruct_boundary_flux_from_coils (:162-267), in its expressions."""
+    frac = float(np.mean(_points_inside_polygon(obs, lim)))
+    return {"limiter_points": lim, "limiter_point_count": int(lim.shape[0]),
+            "min_limiter_distance_m": float(np.min(np.linalg.norm(lim[:, None, :] - obs[None, :, :], axis=2))),
+            "boundary_containment_fraction": frac, "boundary_containment_pass": bool(frac >= 1.0)}
+
+
+def _x_pair_symmetric(x_points: np.ndarray, axis: np.ndarray) -> np.ndarray:
+    """Per sample, the reference's condition for x_point_pair_symmetry_abs_error: two X-points at one R, mirrored about
+    the axis height.  x_points (B, 2, 2), axis (B, 2) -> (B,) bool."""
+    return ((np.abs(x_points[:, 0, 0] - x_points[:, 1, 0]) <= 1.0e-9)
+            & (np.abs(x_points[:, 0, 1] + x_points[:, 1, 1] - 2.0 * axis[:, 1]) <= 1.0e-9))
+
+
 def _kernel_boundary_points(kernel: Any) -> np.ndarray:
     return _wall_contour(kernel)[0]
 

@@ -686,7 +686,9 @@ class BatchedFusionKernel(_GridMixin):
                             max_outer_iter: int = 20, tol: float = 1e-4, plasma_wall: bool = False,
                             wall_mu0: float = _MU0_SI, psi0=None, batch: int | None = None, to_host: bool = True,
                             out: dict | None = None, optimize_shape: bool = False, target_points=None,
-                            target_values=None, current_limits=None, tikhonov_alpha: float = 1e-4) -> dict[str, Any]:
+                            target_values=None, current_limits=None, tikhonov_alpha: float = 1e-4,
+                            reconstruct_boundary: bool = False, limiter_points=None, axis_point=None,
+                            x_points=None) -> dict[str, Any]:
         """``FusionKernel.solve_free_boundary(coils, max_outer_iter, tol, optimize_shape, tikhonov_alpha)``
         (fusion_kernel_free_boundary.py:623-739) for B independent equilibria in one device-resident outer loop.
 
@@ -709,7 +711,17 @@ class BatchedFusionKernel(_GridMixin):
         arrays, ``target_flux`` / ``achieved_flux`` (B, P)) plus ``fit_fallback`` (B,): the fit failed (non-finite
         target) and the clipped prior currents were kept, as the reference does.  Without ``target_points`` the call is
         the ``optimize_shape=False`` solve, like the reference's.
+
+        ``reconstruct_boundary=True`` ends the call with the reference's wall-contour check (:708-739), on the device for
+        the whole batch: the result gains ``boundary_reconstruction`` (``reconstruct_boundary_flux_from_coils`` on the
+        wall contour with the final currents, plus ``limiter_points``, ``axis_point`` and ``x_points``, shared or per
+        sample) and ``vacuum_boundary_abs_error`` (B,), its max_abs_error.  The target is the flux the loop imposed on the
+        wall in each sample's last outer iteration (the reference's psi_ext there): the coil flux (of the final currents
+        with ``optimize_shape``), or with ``plasma_wall`` alone the wall ring of the final psi (coil plus plasma wall
+        flux, to the rounding of the last Picard under-relaxation).  Integer ``turns`` are then required.
         """
+        if not reconstruct_boundary and not (limiter_points is None and axis_point is None and x_points is None):
+            raise ValueError("limiter_points, axis_point and x_points need reconstruct_boundary=True.")
         if max_outer_iter < 1:
             raise ValueError("max_outer_iter must be >= 1.")
         if not np.isfinite(tol) or tol < 0.0:
@@ -732,6 +744,10 @@ class BatchedFusionKernel(_GridMixin):
         shape = bool(optimize_shape) and target_points is not None
         spec = self._shape_spec(B, tr, target_points, target_values, current_limits, tikhonov_alpha) if shape else None
         t0 = time.time()
+        bspec = None
+        if reconstruct_boundary:
+            from .free_boundary import _wall_contour
+            bspec = self._boundary_spec(B, tr, _wall_contour(self)[0], limiter_points, axis_point, x_points)
         psi_in = None if psi0 is None else D.to_device(np.asarray(psi0, dtype=np.float64).reshape(B, self.NZ, self.NR),
                                                        self.device)
         kw = dict(max_outer_iter=max_outer_iter, tol=tol, plasma_wall=plasma_wall, wall_mu0=wall_mu0, psi_out=psi_in,
@@ -746,6 +762,16 @@ class BatchedFusionKernel(_GridMixin):
         else:
             w = cc * tr[None, :]  # I * turns (fusion_kernel_free_boundary.py:88-92)
             dev = self.solve_free_boundary_device(D.to_device(w, self.device), ipd, pedd, **kw)
+        if bspec is not None:
+            # the reference's psi_ext after its loop: the coil flux (psi_ext; with shape steps that of the final
+            # currents), or with the plasma wall flux the ring the last outer iteration imposed on psi, which only the
+            # Picard under-relaxation (1-a) x + a x has touched since (rounding)
+            field = dev["psi"] if plasma_wall and not shape else dev["psi_ext"]
+            bdev = self._boundary_call(bspec, dev["currents"] if shape else D.to_device(cc, self.device), field, 3)
+            from .free_boundary import _wall_contour
+            _, iz, ir = _wall_contour(self)
+            idx = D.torch_mod().as_tensor(iz * self.NR + ir, device=field.device)
+            ring = field.reshape(B, -1)[:, idx].cpu().numpy()
         res = self.unpack_summary(dev["summary"].cpu().numpy())
         fb = dev["fb_summary"].cpu().numpy()
         res.update({"outer_iterations": fb[:, 0].astype(np.int64), "final_diff": fb[:, 1],
@@ -753,6 +779,9 @@ class BatchedFusionKernel(_GridMixin):
         if shape:
             res["coil_currents"] = dev["currents"].cpu().numpy()
             res["shape_optimization"] = self._shape_report(spec, dev["shape_out"].cpu().numpy())
+        if bspec is not None:
+            br = res["boundary_reconstruction"] = self._boundary_report(bspec, bdev, ring)
+            res["vacuum_boundary_abs_error"] = br["max_abs_error"]
         self._fields_to_host(res, dev, to_host, out)
         res["wall_time_s"] = time.time() - t0
         return res
@@ -1027,6 +1056,220 @@ class BatchedFusionKernel(_GridMixin):
         if events is not None:
             events[1].record()
         return {"currents": cur, "residual": res, "weighted_residual": wres, "stats": stats}
+
+    # -- wall-contour boundary reconstruction ------------------------------------------------------------
+    def _boundary_spec(self, B: int, turns, boundary_points, limiter_points, axis_point, x_points) -> dict[str, Any]:
+        """Check the reconstruction inputs with the reference's messages (free_boundary.py) and the device's limits, and
+        compute the host geometry once (no device work).  An axis (B, 2) or X-points (B, X, 2) make both per sample."""
+        from .free_boundary import _limiter_geometry, _points, _x_pair_symmetric
+        cfg_coils = self.cfg["coils"]
+        n = len(cfg_coils)
+        if n < 1:
+            raise ValueError("CoilSet.positions must contain at least one coil.")
+        tr = np.array([c.get("turns", 1) for c in cfg_coils], dtype=np.float64) if turns is None \
+            else np.asarray(turns, dtype=np.float64).reshape(-1)
+        if tr.shape[0] != n or not np.all(np.isfinite(tr)) or np.any(tr < 1) or np.any(tr != np.round(tr)):
+            raise ValueError("turns must be positive integers.")
+        obs = np.ascontiguousarray(_points(boundary_points, "boundary_points"))
+        if obs.shape[0] > 4096:
+            raise ValueError("boundary reconstruction supports at most 4096 boundary points on the device.")
+        lim = None
+        if limiter_points is not None:
+            lim = np.ascontiguousarray(_points(limiter_points, "limiter_points"))
+            if lim.shape[0] > 4096:
+                raise ValueError("boundary reconstruction supports at most 4096 limiter points on the device.")
+        per = False
+        ax = None
+        if axis_point is not None:
+            a = np.asarray(axis_point, dtype=np.float64)
+            if a.size == 2:
+                ax = _points(a.reshape(1, 2), "axis_point")[0]
+            elif a.shape == (B, 2):
+                ax, per = _points(a, "axis_point"), True
+            else:
+                raise ValueError(f"axis_point must have shape (2,) or ({B}, 2).")
+        xo = None
+        if x_points is not None:
+            x = np.asarray(x_points, dtype=np.float64)
+            if x.ndim == 3:
+                if x.shape[0] != B or x.shape[1] < 1 or x.shape[2] != 2:
+                    raise ValueError(f"x_points must have shape (n_points, 2) or ({B}, n_points, 2).")
+                _points(x.reshape(-1, 2), "x_points")
+                xo, per = x, True
+            else:
+                xo = _points(x, "x_points")
+            if xo.shape[-2] > 64:
+                raise ValueError("boundary reconstruction supports at most 64 X-points on the device.")
+        for p in (obs, lim, ax, xo):
+            if p is not None and np.any(p[..., 0] <= 0.0):
+                raise ValueError("observation radii must be positive.")
+        X = 0 if xo is None else int(xo.shape[-2])
+        # the C entry reads the point arrays in storage order; per sample, both the axis and the X-points are
+        if ax is not None:
+            ax = np.ascontiguousarray(np.broadcast_to(ax, (B, 2)) if per else ax)
+        if xo is not None:
+            xo = np.ascontiguousarray(np.broadcast_to(xo, (B, X, 2)) if per else xo)
+        pos = [(c["r"], c["z"]) for c in cfg_coils]
+        tri = np.ascontiguousarray(tr.astype(np.int32))
+        geo: dict[str, Any] = {"boundary_points": obs, "point_count": int(obs.shape[0]), "coil_count": n,
+                               "limiter_point_count": 0, "min_limiter_distance_m": None, "axis_point": ax,
+                               "x_point_count": X, "x_point_pair_symmetry_abs_error": None}
+        if lim is not None:
+            geo.update(_limiter_geometry(obs, lim))
+        if xo is not None:
+            geo["x_points"] = xo
+        sym = None
+        if ax is not None and X == 2:
+            ok = _x_pair_symmetric(xo if per else xo[None], ax if per else ax[None])
+            if ok.any():
+                sym = np.broadcast_to(ok, (B,)) if not per else ok
+        return {"B": B, "per_sample": per, "coil_rz": np.ascontiguousarray(np.asarray(pos, dtype=np.float64).reshape(n, 2)),
+                "turns": tri, "points": obs, "limiter": lim, "axis": ax, "xpoints": xo, "X": X, "symmetric": sym,
+                "geometry": geo}
+
+    def _boundary_call(self, spec, currents_dev, target_dev, mode: int, events=None) -> dict[str, Any]:
+        """One gsb_boundary_flux launch; mode = target_mode of gsb_boundary_params.  "response" is the boundary columns
+        (n_coils, N) of the M the entry built in its workspace and used."""
+        lib = _lib.load()
+        dp = ctypes.POINTER(ctypes.c_double)
+        B, n = spec["B"], spec["coil_rz"].shape[0]
+        N = spec["points"].shape[0]
+        L = 0 if spec["limiter"] is None else spec["limiter"].shape[0]
+        A, X = int(spec["axis"] is not None), spec["X"]
+        bp = _lib.gsb_boundary_params()
+        bp.n_coils, bp.coil_rz = n, spec["coil_rz"].ctypes.data_as(dp)
+        bp.turns = spec["turns"].ctypes.data_as(ctypes.POINTER(ctypes.c_int))
+        bp.n_points, bp.points = N, spec["points"].ctypes.data_as(dp)
+        bp.n_limiter, bp.limiter = L, None if not L else spec["limiter"].ctypes.data_as(dp)
+        bp.has_axis, bp.axis = A, None if not A else spec["axis"].ctypes.data_as(dp)
+        bp.n_xpoints, bp.xpoints = X, None if not X else spec["xpoints"].ctypes.data_as(dp)
+        bp.per_sample, bp.target_mode = int(spec["per_sample"]), int(mode)
+        if mode == 3:
+            bp.nz, bp.nr = self.NZ, self.NR
+            r_ax, z_ax = np.ascontiguousarray(self.R, dtype=np.float64), np.ascontiguousarray(self.Z, dtype=np.float64)
+            bp.r_axis, bp.z_axis = r_ax.ctypes.data_as(dp), z_ax.ctypes.data_as(dp)
+        null = ctypes.c_void_p()
+        need = ctypes.c_longlong(0)
+        _lib.check(lib.gsb_boundary_flux(ctypes.byref(bp), null, null, null, null, null, null, ctypes.byref(need), B,
+                                         null), "gsb_boundary_flux")
+        work = D.empty(((need.value + 7) // 8,), self.device)
+        need.value = work.numel() * 8
+        flux, stats = D.empty((B, N + L + A + X), self.device), D.empty((B, 5), self.device)
+        res = D.empty((B, N), self.device) if mode else None
+        if events is not None:
+            events[0].record()
+        _lib.check(lib.gsb_boundary_flux(ctypes.byref(bp), D.ptr(currents_dev), null if not mode else D.ptr(target_dev),
+                                         D.ptr(flux), null if res is None else D.ptr(res), D.ptr(stats), D.ptr(work),
+                                         ctypes.byref(need), B, D.stream_ptr()), "gsb_boundary_flux")
+        if events is not None:
+            events[1].record()
+        ncol = N + L + (B if spec["per_sample"] else 1) * (A + X)
+        return {"flux": flux, "residual": res, "stats": stats, "response": work[:n * ncol].view(n, ncol)[:, :N]}
+
+    def _boundary_report(self, spec, dev, target) -> dict[str, Any]:
+        """The reference's reconstruct_boundary_flux_from_coils dict over the batch; raises ValueError naming the samples
+        with non-finite boundary flux or target."""
+        flux, st = dev["flux"].cpu().numpy(), dev["stats"].cpu().numpy()
+        flags = st[:, 4].astype(np.int64)
+        bad = np.flatnonzero(flags & 1)
+        if bad.size:
+            raise ValueError(f"reconstructed boundary flux contains non-finite values in samples {bad.tolist()}")
+        bad = np.flatnonzero(flags & 2)
+        if bad.size:
+            raise ValueError(f"target_flux must contain finite values only: samples {bad.tolist()}")
+        N = spec["points"].shape[0]
+        L = 0 if spec["limiter"] is None else spec["limiter"].shape[0]
+        A, X = int(spec["axis"] is not None), spec["X"]
+        d = dict(spec["geometry"])
+        resp = d["response_matrix"] = dev["response"].cpu().numpy()
+        d["response_rank"] = int(np.linalg.matrix_rank(resp))
+        d.update({"reconstructed_flux": flux[:, :N], "limiter_flux": flux[:, N:N + L], "axis_flux": None,
+                  "x_point_flux": flux[:, N + L + A:], "x_point_flux_span": None})
+        if A:
+            d["axis_flux"] = flux[:, N + L]
+        if X:
+            d["x_point_flux_span"] = st[:, 2].copy()
+        if spec["symmetric"] is not None:
+            d["x_point_pair_symmetry_abs_error"] = np.where(spec["symmetric"], st[:, 3], np.nan)
+        if target is not None:
+            d.update({"target_flux": target, "residual": dev["residual"].cpu().numpy(), "rmse": st[:, 0].copy(),
+                      "max_abs_error": st[:, 1].copy()})
+        return d
+
+    def reconstruct_boundary_flux_from_coils(self, coil_currents=None, *, boundary_points, limiter_points=None,
+                                             axis_point=None, x_points=None, target_flux=None,
+                                             turns=None) -> dict[str, Any]:
+        """``FusionKernel.reconstruct_boundary_flux_from_coils`` (fusion_kernel_free_boundary.py:162-267) for B coil-current
+        vectors in one device call (gsb_boundary_flux).
+
+        coil_currents (B, n_coils) | (n_coils,) (a batch of one) | None (config currents) in amperes; turns (n_coils,) |
+        None = config turns; axis_point (2,) or (B, 2) and x_points (X, 2) or (B, X, 2): shared or per sample;
+        target_flux (N,) or (B, N).  Returns the reference's keys.  Per-sample values have a leading batch axis:
+        reconstructed_flux (B, N), limiter_flux (B, L), axis_flux (B,), x_point_flux (B, X), x_point_flux_span (B,),
+        residual (B, N), rmse and max_abs_error (B,).  The geometry-only values are computed once on the host.
+        x_point_pair_symmetry_abs_error is None where the reference gives None for every sample, otherwise (B,) with NaN
+        for the samples whose X-point pair is not mirrored about their axis.  Each flux is sum_c M[c][p] I_c in coil
+        order, so a sample's values do not depend on the batch.  Raises ValueError naming the samples whose boundary
+        flux is not finite.
+        """
+        from .free_boundary import _points, _vector
+        n = len(self.cfg["coils"])
+        cur = np.array([[c.get("current", 0.0) for c in self.cfg["coils"]]], dtype=np.float64) if coil_currents is None \
+            else np.asarray(coil_currents, dtype=np.float64)
+        if cur.ndim == 1:
+            cur = cur[None, :]
+        if cur.ndim != 2 or cur.shape[0] < 1 or cur.shape[1] != n:
+            raise ValueError(f"currents must have length {n}.")
+        if not np.all(np.isfinite(cur)):
+            raise ValueError("currents must contain finite values only.")
+        B = cur.shape[0]
+        N = _points(boundary_points, "boundary_points").shape[0]
+        t = None
+        if target_flux is not None:
+            t = np.asarray(target_flux, dtype=np.float64)
+            if t.ndim <= 1:
+                t = _vector(t, "target_flux", N)
+            elif t.shape != (B, N):
+                raise ValueError(f"target_flux must have length {N}.")
+            elif not np.all(np.isfinite(t)):
+                raise ValueError("target_flux must contain finite values only.")
+        spec = self._boundary_spec(B, turns, boundary_points, limiter_points, axis_point, x_points)
+        dev = self._boundary_call(spec, D.to_device(cur, self.device), None if t is None else D.to_device(t, self.device),
+                                  0 if t is None else (1 if t.ndim == 1 else 2))
+        return self._boundary_report(spec, dev, t)
+
+    def reconstruct_boundary_flux_device(self, currents_dev, *, boundary_points, limiter_points=None, axis_point=None,
+                                         x_points=None, target_dev=None, target_field=None, turns=None,
+                                         events=None) -> dict[str, Any]:
+        """Device-resident boundary reconstruction (gsb_boundary_flux): currents_dev (B, n_coils) CUDA float64 in amperes;
+        the target is target_dev (N,) | (B, N), or the wall contour of target_field (B, nz, nr) (boundary_points must then
+        be that contour, ``_wall_contour``), or none; other keywords as ``reconstruct_boundary_flux_from_coils``.
+        Returns device tensors flux (B, N + L + A + X) (boundary, limiter, axis, X-point flux in that order), residual
+        (B, N) (None without a target), response (n_coils, N) (the boundary columns of the M the flux was summed over, a
+        view of the call's workspace) and stats (B, 5): rmse, max |residual|, X-point flux span, |xf0 - xf1|, flags
+        (1: a boundary flux is not finite, 2: a target value is not finite); NaN where a value does not apply."""
+        from .free_boundary import _points, _wall_contour
+        torch = D.torch_mod()
+        B, n = int(currents_dev.shape[0]), len(self.cfg["coils"])
+        obs = _points(boundary_points, "boundary_points")
+        N = obs.shape[0]
+        if target_dev is not None and target_field is not None:
+            raise ValueError("give target_dev or target_field, not both.")
+        checks = [(currents_dev, [(B, n)], "currents_dev")]
+        mode, tgt = 0, None
+        if target_dev is not None:
+            checks.append((target_dev, [(N,), (B, N)], "target_dev"))
+            mode, tgt = (1 if target_dev.ndim == 1 else 2), target_dev
+        elif target_field is not None:
+            checks.append((target_field, [(B, self.NZ, self.NR)], "target_field"))
+            if not np.array_equal(obs, _wall_contour(self)[0]):
+                raise ValueError("the wall-contour target needs the wall contour of the grid as boundary points.")
+            mode, tgt = 3, target_field
+        for t, shapes, name in checks:
+            if tuple(t.shape) not in shapes or t.dtype != torch.float64 or not t.is_contiguous() or not t.is_cuda:
+                raise ValueError(f"{name} must be a contiguous CUDA float64 tensor of shape {' or '.join(map(str, shapes))}.")
+        spec = self._boundary_spec(B, turns, boundary_points, limiter_points, axis_point, x_points)
+        return self._boundary_call(spec, currents_dev, tgt, mode, events)
 
     def solve_device(self, w_dev, ip_dev, ped_dev=None, *, want_history: bool = False, psi_out=None,
                      jphi_out=None, events=None) -> dict[str, Any]:
